@@ -4,6 +4,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this backend (libraytracing_cuda.so)
   python bench.py --impl reference --steps K --warmup W    # the reference algorithm on the host cores
+  python bench.py --dump-outputs DIR                       # + the planes of the last timed step as DIR/<plane>.npy
 
 A step = one full render of the frame (one pass of the hot path over one batch of synthetic-free, fixed
 input: the scene fixture committed under tests/golden/scenes). See DESIGN.md "Measurement".
@@ -18,6 +19,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 WORKLOADS = {
     # name: (fixture, width, height, spp, depth, light samples)
@@ -126,6 +128,28 @@ class ClockSampler(threading.Thread):
                 "samples": len(self.rows), "source": self.source}
 
 
+DUMP_BYTES = 64_000_000
+DUMP_SAMPLE_PIXELS = 1 << 20   # x at most 13 float32 channels, + their float64 indices: 63 MB
+
+
+def dump_outputs(path, planes):
+    """--dump-outputs: the planes the timed path handed back in its last step (rank 0 after the combine: the full frame) as
+    <path>/<plane>.npy, float32 [H, W, C]. When the frame's planes come to more than DUMP_BYTES together, every plane is written
+    at the same fixed, seeded sample of DUMP_SAMPLE_PIXELS pixels instead ([N, C], in raster order), and pixel_index.npy
+    (float64, exact) holds their flat y * W + x indices. One-channel planes (mip_level, debug_depth) keep their channel axis,
+    [H, W, 1], where a RenderOutput holds them as [H, W]."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {name: t.cpu().numpy() for name, t in planes.items()}
+    h, w = next(iter(arrays.values())).shape[:2]
+    if sum(a.nbytes for a in arrays.values()) > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(42).choice(h * w, size=DUMP_SAMPLE_PIXELS, replace=False))
+        arrays = {name: a.reshape(h * w, -1)[idx] for name, a in arrays.items()}
+        arrays["pixel_index"] = idx.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def peaks():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(path):
@@ -165,7 +189,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--tile-size", type=int, default=0, help="tile edge of the multi-GPU deal (0 = per workload: 64 for C5, else 16)")
     ap.add_argument("--partition", default="tiles", choices=["tiles", "samples"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the planes of the last timed step to DIR/<plane>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -241,7 +268,7 @@ def main():
             red = e0.elapsed_time(e1)
             ms += red
             stats = dict(stats, reduce_ms=red)
-        return ms, stats
+        return ms, stats, planes
 
     for _ in range(args.warmup):
         one_step()
@@ -252,7 +279,7 @@ def main():
     total_ms, agg = 0.0, {}
     wall0 = time.time()
     for _ in range(args.steps):
-        ms, stats = one_step()
+        ms, stats, planes = one_step()
         total_ms += ms
         for k in ("samples", "primary_rays", "bounce_rays", "shadow_rays", "primary_rays_culled", "kernel_launches", "extend_launches", "shade_launches",
                   "shadow_launches", "extend_ms", "shade_ms", "shadow_ms", "gather_ms", "other_ms", "render_ms", "reduce_ms"):
@@ -260,6 +287,8 @@ def main():
     sync_all()
     wall = time.time() - wall0
     clocks.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, planes)
     t = torch.tensor([total_ms], dtype=torch.float64, device=f"cuda:{local_rank}")
     cnt = torch.tensor([agg["samples"], agg["primary_rays"] + agg["bounce_rays"] + agg["shadow_rays"], agg["kernel_launches"], agg["primary_rays_culled"]],
                        dtype=torch.float64, device=f"cuda:{local_rank}")
@@ -278,7 +307,7 @@ def main():
     # ---- end to end through the public API with HOST buffers: rc.render(scene, settings) per step =
     # context + scene upload (H2D) + device BVH build + render + D2H of the frame (raytracing_cpu::render also
     # builds its acceleration structures inside every call, lib.rs:655)
-    e2e_steps = max(1, min(args.steps, 2))
+    e2e_steps = args.steps
     holder = sc.to_desc(own_arrays=True)
     h2d = int(holder.geometry_bytes + holder.image_bytes.nbytes)
     e2e_each = []

@@ -41,24 +41,21 @@ _lib_path = LIB_PATH
 def use_native_build() -> str:
     """The CPU-baseline build (bench.py): the same oracle.cpp compiled `-O3 -march=native` ON THE HOST IT RUNS ON
     (BASELINE.md / SURVEY 8d), still -ffp-contract=off so its pixels are the portable build's. Kept apart from liboracle.so,
-    which is built -O2 for any x86-64 host because the prebuilt file travels from the build container to the GPU box."""
+    which is built -O2 for any x86-64 host because the prebuilt file may be loaded on another host than the one that built it.
+    The native library goes to a temporary directory of this process (removed at exit), so that the source tree may be read-only."""
     global _lib, _lib_path
-    import hashlib
-    import platform
-    cpu = ""
-    try:
-        cpu = next(l for l in open("/proc/cpuinfo") if l.startswith("model name"))
-    except Exception:
-        cpu = platform.processor()
-    tag = hashlib.sha1((cpu + platform.machine()).encode()).hexdigest()[:10]
-    path = os.path.join(_HERE, f"liboracle_native_{tag}.so")
+    import atexit
+    import shutil
+    import tempfile
+    if _lib_path != LIB_PATH:   # already built by this process
+        return _lib_path
+    tmp = tempfile.mkdtemp(prefix="raytracing_cuda_oracle_")
+    atexit.register(shutil.rmtree, tmp, ignore_errors=True)
+    path = os.path.join(tmp, "liboracle_native.so")
     src = os.path.join(_HERE, "oracle.cpp")
-    hdr = os.path.join(os.path.dirname(_HERE), "include", "rtcuda.h")
-    if not os.path.exists(path) or os.path.getmtime(path) < max(os.path.getmtime(src), os.path.getmtime(hdr)):
-        subprocess.check_call(["g++", "-O3", "-march=native", "-std=c++17", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-pthread",
-                               "-shared", "-o", path, src])
-    if path != _lib_path:
-        _lib, _lib_path = None, path
+    subprocess.check_call(["g++", "-O3", "-march=native", "-std=c++17", "-fPIC", "-ffp-contract=off", "-fno-fast-math", "-pthread",
+                           "-shared", "-o", path, src])
+    _lib, _lib_path = None, path
     return path
 
 

@@ -216,6 +216,64 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert d["config"]["workload"].startswith("C2")
 
 
+def _bench_module(monkeypatch):
+    import importlib.util
+    import sys
+    monkeypatch.setattr(sys, "dont_write_bytecode", sys.dont_write_bytecode)   # restored after the test (bench.py sets it)
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_dump_outputs_whole_or_sampled(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: whole planes while they fit DUMP_BYTES, else every plane at the same fixed sample of pixels"""
+    import torch
+    bench = _bench_module(monkeypatch)
+    planes = {"beauty": torch.rand(48, 64, 3), "debug_depth": torch.rand(48, 64, 1)}
+    bench.dump_outputs(str(tmp_path / "whole"), planes)
+    assert sorted(os.listdir(tmp_path / "whole")) == ["beauty.npy", "debug_depth.npy"]
+    for name, t in planes.items():
+        assert np.array_equal(np.load(tmp_path / "whole" / f"{name}.npy"), t.numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096)
+    monkeypatch.setattr(bench, "DUMP_SAMPLE_PIXELS", 100)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), planes)
+    idx = np.load(tmp_path / "a" / "pixel_index.npy")
+    assert idx.dtype == np.float64 and len(idx) == 100 and (np.diff(idx) > 0).all()
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "pixel_index.npy"))
+    for name, t in planes.items():
+        a = np.load(tmp_path / "a" / f"{name}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, t.numpy().reshape(48 * 64, -1)[idx.astype(np.int64)])
+
+
+def test_bench_rejects_zero_steps():
+    import subprocess
+    import sys
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=60)
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
+@pytest.mark.gpu
+def test_bench_dumps_the_frame_of_the_timed_steps(rc, tmp_path, monkeypatch):
+    """bench.py --steps K --dump-outputs DIR: K timed steps (and K end-to-end calls), and DIR/beauty.npy is the frame the
+    renderer returns for the same workload"""
+    import json
+    import subprocess
+    import sys
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "C2", "--steps", "2", "--warmup", "1",
+                          "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][0])
+    assert d["steps"] == 2 and d["e2e"]["steps"] == 2 and len(d["e2e"]["breakdown"]) == 2
+    assert sorted(os.listdir(tmp_path)) == ["beauty.npy"]
+    sc, st = _bench_module(monkeypatch).load_workload("C2")
+    with rc.CudaRenderer(sc) as r:
+        frame = r.render(st).beauty
+    assert np.array_equal(np.load(tmp_path / "beauty.npy"), frame)
+    assert d["config"]["workload"].startswith("C2")
+
+
 def test_integration_patch_applies(tmp_path):
     """integration/reference.patch is a real diff against the reference tree: it applies cleanly to copies of the files it
     names (only where /root/reference exists: the GPU box does not have it), and the Rust crate only calls entry points and

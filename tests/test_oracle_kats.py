@@ -1,11 +1,12 @@
 """Pins the CPU oracle against every known-answer test the reference holds for the path (SURVEY §8c) and
 against published vectors of the third-party generators it restates."""
 import ctypes as C
+import os
 
 import numpy as np
 import pytest
 
-from conftest import load_scene
+from conftest import GOLDEN, load_scene
 
 
 def fa(v):
@@ -63,36 +64,29 @@ def test_fxhash_structure(oracle):
     assert oracle.lib().oracle_fxhash_u32x3(3, 5, 7) == rotl(h, 26)
 
 
-def test_fxhasher_constants_against_compiled_rustc_hash():
+def test_fxhasher_constants_against_compiled_rustc_hash(oracle):
     """Evidence for the two constants the reference's tests do not pin (SURVEY appendix C: multiplier K and the rotate of
-    `finish`): Rust extension modules in this image that link rustc-hash 2.x (tokenizers, tiktoken, outlines_core) carry K as a
-    64-bit immediate, and the `rol r64, 26` of `finish()` follows it. rustc-hash 2.0.0 rotated by 20; 1.x used another K."""
-    import glob
-    import importlib.util
+    `finish`): Rust extension modules that link rustc-hash 2.x (tokenizers 0.22.2, tiktoken 0.12.0, outlines_core 0.2.14) carry K
+    as a 64-bit immediate, and the `rol r64, 26` of `finish()` follows it. rustc-hash 2.0.0 rotated by 20; 1.x used another K.
+    The machine code that follows each K in those modules is stored in tests/golden/rustc_hash_k_windows.npz
+    (tests/golden/make_rustc_hash_windows.py). The oracle's FxHasher must use the K and the rotate found there."""
     K = bytes.fromhex("c5a9622eea7a35f1")           # 0xf1357aea2e62a9c5, little endian
-    files = []
-    for mod in ("tiktoken", "tokenizers", "outlines_core"):
-        spec = importlib.util.find_spec(mod)
-        if spec and spec.submodule_search_locations:
-            for d in spec.submodule_search_locations:
-                files += glob.glob(d + "/*.so")
-    if not files:
-        pytest.skip("no Rust extension module with rustc-hash in this environment")
+    z = np.load(os.path.join(GOLDEN, "rustc_hash_k_windows.npz"))
+    assert {s.split(":")[0].split()[0] for s in z["sources"]} == {"tiktoken", "tokenizers", "outlines_core"}
     rol26 = rol20 = with_k = 0
-    for f in files:
-        data = open(f, "rb").read()
-        i = data.find(K)
-        while i >= 0:
-            with_k += 1
-            window = data[i + 8:i + 96]
-            for j in range(len(window) - 3):   # rol r64, imm8 = REX.W(48/49) C1 /0 ib
-                if window[j] in (0x48, 0x49) and window[j + 1] == 0xC1 and 0xC0 <= window[j + 2] <= 0xC7:
-                    rol26 += window[j + 3] == 26
-                    rol20 += window[j + 3] == 20
-            i = data.find(K, i + 8)
-    if not with_k:
-        pytest.skip("rustc-hash 2.x not linked into the Rust extension modules found")
+    for row in z["windows"]:
+        assert bytes(row[:8]) == K
+        with_k += 1
+        window = bytes(row[8:])
+        for j in range(len(window) - 3):   # rol r64, imm8 = REX.W(48/49) C1 /0 ib
+            if window[j] in (0x48, 0x49) and window[j + 1] == 0xC1 and 0xC0 <= window[j + 2] <= 0xC7:
+                rol26 += window[j + 3] == 26
+                rol20 += window[j + 3] == 20
     assert rol26 >= 5 and rol20 == 0, (with_k, rol26, rol20)
+    k, m = int.from_bytes(K, "little"), (1 << 64) - 1
+    for x in (1, 42, 0xdeadbeef, m):
+        h = (x * k) & m
+        assert oracle.lib().oracle_fxhash_u64(x) == ((h << 26) | (h >> 38)) & m, x
 
 
 def test_uniform_f32_is_24bit(oracle, rc):

@@ -5,7 +5,7 @@ CSRC := $(PKG)/csrc
 NVCCFLAGS := -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -Xcompiler -fvisibility=hidden $(NVCCFLAGS_EXTRA)
 HDRS := $(wildcard $(CSRC)/*.h) $(CSRC)/kernels.cuh include/rtcuda.h
 
-all: $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so oracle_ref
+all: $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so oracle_ref
 
 # the reference's own C++ device headers compiled for the host (checker of the oracle; no-op when /root/reference is absent)
 .PHONY: oracle_ref
@@ -38,5 +38,9 @@ oracle/liboracle.so: oracle/oracle.cpp include/rtcuda.h
 tests/hostsim/libhostsim.so: tests/hostsim/hostsim.cpp $(HDRS)
 	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
 
+# the scene-update refit on the CPU (includes hostsim.cpp)
+tests/hostsim/libhostsim_update.so: tests/hostsim/hostsim_update.cpp tests/hostsim/hostsim.cpp $(HDRS)
+	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
+
 clean:
-	rm -rf build $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so
+	rm -rf build $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so

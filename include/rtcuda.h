@@ -38,7 +38,7 @@ extern "C" {
 #define RTCUDA_API __attribute__((visibility("default")))
 #endif
 
-#define RTCUDA_ABI_VERSION 3u
+#define RTCUDA_ABI_VERSION 4u
 #define RTCUDA_MAX_DEVICES 8u
 #define RTCUDA_NONE 0xffffffffu
 
@@ -349,6 +349,12 @@ typedef struct rtcuda_stats {
      * scene bounds (raster rectangle of the projected bounds; only without an environment light, pinhole / orthographic
      * cameras). Their samples are counted in primary_rays and primary_rays_culled like the per-sample culls. */
     uint64_t pixels_dropped;
+    /* ABI v4 */
+    double update_ms;                 /* device time of the last rtcuda_scene_update */
+    /* SAH cost of the current wide tree, (A(root) + sum over inner children A(c) + sum over leaf children A(c) * |c|) / A(root)
+     * with A the surface area of the child's float box (node and primitive cost 1); 0 until the first update computed it. */
+    double bvh_sah_cost;
+    uint64_t bvh_last_update;         /* last rtcuda_scene_update: 0 nothing changed, 1 camera / lights only, 2 refit, 3 rebuild */
 } rtcuda_stats;
 
 typedef struct rtcuda_ctx rtcuda_ctx;
@@ -363,6 +369,22 @@ RTCUDA_API void rtcuda_shutdown(rtcuda_ctx* ctx);
  * builds the mip pyramids for trilinear textures and the 8-wide BVH on the device. */
 RTCUDA_API rtcuda_status rtcuda_scene_upload(rtcuda_ctx* ctx, const rtcuda_scene_desc* desc, rtcuda_scene** out_scene);
 RTCUDA_API void rtcuda_scene_release(rtcuda_scene* scene);
+
+/* Moves what the caller moved: reads desc->camera (raster size and kind must be unchanged),
+ * desc->instances[i].object_to_world (forward + inverse), and desc->lights[i]
+ * position_or_direction / intensity_or_radiance / light_to_world.
+ * desc must have the topology of the uploaded scene:
+ *   - same shape / instance / light / material / texture / image counts;
+ *   - same instances[i].shape;
+ *   - same lights[i].kind and .shape.
+ * Geometry arrays, shapes, materials, textures and images are NOT read (may be NULL).
+ * On a mismatch: RTCUDA_ERR_INVALID_ARGUMENT and the scene is left untouched.
+ * Blocks until the device scene is updated. Multi-device scenes are updated on every GPU.
+ * The library compares desc against what it holds and does only the work the differences need: new kernel constants for
+ * the camera and the lights; for moved instances a refit of the wide BVH on the device (primitive slots recomputed in
+ * place, node boxes re-fitted level by level), or a rebuild from the resident geometry when the refit's SAH cost grew too
+ * far over the built tree's. Frames rendered afterwards equal the frames of a fresh upload of desc, bit for bit. */
+RTCUDA_API rtcuda_status rtcuda_scene_update(rtcuda_scene* scene, const rtcuda_scene_desc* desc);
 
 /* The path-state arena of a released scene (multi-GB: batches are sized for HBM) is parked per process and reused by
  * the next scene on the same device, so back-to-back one-shot renders do not pay for mapping device memory again.

@@ -367,13 +367,17 @@ fn settings_to_c(s: &RaytracerSettings) -> ffi::rtcuda_settings {
     c
 }
 
-struct Uploaded {
+/// A scene uploaded to the device (context + device BVH) that can be rendered repeatedly and moved in place with
+/// [`CudaScene::update`]: what a viewer keeps between frames.
+pub struct CudaScene {
     ctx: *mut ffi::rtcuda_ctx,
     scene: *mut ffi::rtcuda_scene,
+    width: usize,
+    height: usize,
 }
 
-impl Uploaded {
-    fn new(scene: &Scene, backend_settings: &CudaBackendSettings) -> Self {
+impl CudaScene {
+    pub fn new(scene: &Scene, backend_settings: &CudaBackendSettings) -> Self {
         let flat = flatten(scene);
         let mut ctx = ptr::null_mut();
         let mut sc = ptr::null_mut();
@@ -387,11 +391,67 @@ impl Uploaded {
                 panic!("rtcuda_scene_upload failed ({st:?}): {msg}");
             }
         }
-        Uploaded { ctx, scene: sc }
+        CudaScene { ctx, scene: sc, width: scene.camera.raster_width, height: scene.camera.raster_height }
+    }
+
+    /// Moves the camera, the instance transforms and the lights to those of `scene` (`rtcuda_scene_update`): the BVH is
+    /// refitted (or rebuilt) on the device and no geometry is copied again. `scene` must have the uploaded scene's topology
+    /// (same shapes, instance -> shape map, light kinds, materials, textures, raster size and camera kind); otherwise
+    /// RTCUDA_ERR_INVALID_ARGUMENT is returned and the uploaded scene is left as it was.
+    pub fn update(&mut self, scene: &Scene) -> Result<(), String> {
+        let flat = flatten(scene);   // no mesh data is copied: the shapes point at the scene's own Vecs
+        // SAFETY: the desc points into `flat`, which outlives the call; the call blocks until the device scene is updated
+        unsafe {
+            let st = ffi::rtcuda_scene_update(self.scene, &flat.desc);
+            if st != ffi::rtcuda_status::RTCUDA_OK {
+                return Err(CStr::from_ptr(ffi::rtcuda_last_error()).to_string_lossy().into_owned());
+            }
+        }
+        Ok(())
+    }
+
+    /// The frame `render` returns, from the uploaded (and possibly updated) scene
+    pub fn render(&self, raytracer_settings: &RaytracerSettings) -> RenderOutput {
+        let (w, h) = (self.width, self.height);
+        let n = w * h;
+        let o = raytracer_settings.outputs;
+        let mut out = RenderOutput::new(w as u32, h as u32);
+        // only the requested planes are Some (lib.rs:664-677, 685-811)
+        if o.contains(AovFlags::BEAUTY) { out.beauty = Some(vec![Vec3::zero(); n]); }
+        if o.contains(AovFlags::NORMALS) { out.normals = Some(vec![Vec3::zero(); n]); }
+        if o.contains(AovFlags::ALBEDO) { out.albedo = Some(vec![Vec3::zero(); n]); }
+        if o.contains(AovFlags::UV_COORDS) { out.uv = Some(vec![Vec2::zero(); n]); }
+        if o.contains(AovFlags::MIP_LEVEL) { out.mip_level = Some(vec![0.0f32; n]); }
+
+        fn plane<T>(p: &mut Option<Vec<T>>) -> *mut f32 {
+            p.as_mut().map(|v| v.as_mut_ptr() as *mut f32).unwrap_or(ptr::null_mut())
+        }
+        let mut planes = ffi::rtcuda_outputs {
+            width: w as u32,
+            height: h as u32,
+            beauty: plane(&mut out.beauty),   // Vec<Vec3> is 3 packed f32 per pixel (vec3.rs:7-9), row-major y*W+x
+            normals: plane(&mut out.normals),
+            albedo: plane(&mut out.albedo),
+            uv: plane(&mut out.uv),
+            mip_level: plane(&mut out.mip_level),
+            debug_ids: ptr::null_mut(),
+            debug_depth: ptr::null_mut(),
+        };
+        // SAFETY: the planes are alive and sized w*h; the call blocks until they are written
+        unsafe {
+            check(ffi::rtcuda_render(self.scene, &settings_to_c(raytracer_settings), &mut planes), "rtcuda_render");
+            // tail of raytracing_cpu::render (lib.rs:813-854): the device counted the NaN / Inf channels while writing the plane
+            let mut st = ffi::rtcuda_stats::default();
+            ffi::rtcuda_get_stats(self.scene, &mut st);
+            if st.nonfinite_values != 0 {
+                warn_nonfinite(out.beauty.as_ref().unwrap(), w, h);
+            }
+        }
+        out
     }
 }
 
-impl Drop for Uploaded {
+impl Drop for CudaScene {
     fn drop(&mut self) {
         // SAFETY: handles created by rtcuda_init / rtcuda_scene_upload, released exactly once
         unsafe {
@@ -403,43 +463,7 @@ impl Drop for Uploaded {
 
 /// `pub fn render(&Scene, &RaytracerSettings, BackendSettings) -> RenderOutput` (`raytracing-cpu/src/lib.rs:645-649`)
 pub fn render(scene: &Scene, raytracer_settings: &RaytracerSettings, backend_settings: CudaBackendSettings) -> RenderOutput {
-    let (w, h) = (scene.camera.raster_width, scene.camera.raster_height);
-    let n = w * h;
-    let o = raytracer_settings.outputs;
-    let mut out = RenderOutput::new(w as u32, h as u32);
-    // only the requested planes are Some (lib.rs:664-677, 685-811)
-    if o.contains(AovFlags::BEAUTY) { out.beauty = Some(vec![Vec3::zero(); n]); }
-    if o.contains(AovFlags::NORMALS) { out.normals = Some(vec![Vec3::zero(); n]); }
-    if o.contains(AovFlags::ALBEDO) { out.albedo = Some(vec![Vec3::zero(); n]); }
-    if o.contains(AovFlags::UV_COORDS) { out.uv = Some(vec![Vec2::zero(); n]); }
-    if o.contains(AovFlags::MIP_LEVEL) { out.mip_level = Some(vec![0.0f32; n]); }
-
-    let up = Uploaded::new(scene, &backend_settings);
-    fn plane<T>(p: &mut Option<Vec<T>>) -> *mut f32 {
-        p.as_mut().map(|v| v.as_mut_ptr() as *mut f32).unwrap_or(ptr::null_mut())
-    }
-    let mut planes = ffi::rtcuda_outputs {
-        width: w as u32,
-        height: h as u32,
-        beauty: plane(&mut out.beauty),   // Vec<Vec3> is 3 packed f32 per pixel (vec3.rs:7-9), row-major y*W+x
-        normals: plane(&mut out.normals),
-        albedo: plane(&mut out.albedo),
-        uv: plane(&mut out.uv),
-        mip_level: plane(&mut out.mip_level),
-        debug_ids: ptr::null_mut(),
-        debug_depth: ptr::null_mut(),
-    };
-    // SAFETY: the planes are alive and sized w*h; the call blocks until they are written
-    unsafe {
-        check(ffi::rtcuda_render(up.scene, &settings_to_c(raytracer_settings), &mut planes), "rtcuda_render");
-        // tail of raytracing_cpu::render (lib.rs:813-854): the device counted the NaN / Inf channels while writing the plane
-        let mut st = ffi::rtcuda_stats::default();
-        ffi::rtcuda_get_stats(up.scene, &mut st);
-        if st.nonfinite_values != 0 {
-            warn_nonfinite(out.beauty.as_ref().unwrap(), w, h);
-        }
-    }
-    out
+    CudaScene::new(scene, &backend_settings).render(raytracer_settings)
 }
 
 fn warn_nonfinite(beauty: &[Vec3], w: usize, h: usize) {
@@ -465,7 +489,7 @@ fn warn_nonfinite(beauty: &[Vec3], w: usize, h: usize) {
 /// `render_single_pixel` in the `Range<u32>` shape of `raytracing_optix::render_single_pixel`
 /// (`raytracing-optix/src/lib.rs:172-178`); `raytracing_cpu`'s `Option<u32>` form is `index..index + 1`.
 pub fn render_single_pixel(scene: &Scene, raytracer_settings: &RaytracerSettings, x: u32, y: u32, samples: Range<u32>) -> Vec<SinglePixelOutput> {
-    let up = Uploaded::new(scene, &CudaBackendSettings::default());
+    let up = CudaScene::new(scene, &CudaBackendSettings::default());
     let n = samples.end.saturating_sub(samples.start) as usize;
     let mut buf = vec![ffi::rtcuda_pixel_output::default(); n.max(1)];
     // SAFETY: buf holds `n` entries

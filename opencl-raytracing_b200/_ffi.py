@@ -10,7 +10,7 @@ import ctypes as C
 import os
 
 NONE = 0xFFFFFFFF
-ABI_VERSION = 3
+ABI_VERSION = 4
 MAX_DEVICES = 8
 
 # enums (values must match rtcuda.h)
@@ -131,7 +131,8 @@ class Stats(C.Structure):
                 ("upload_ms", C.c_double), ("extend_ms", C.c_double), ("shade_ms", C.c_double),
                 ("shadow_ms", C.c_double), ("other_ms", C.c_double), ("bvh_node_count", C.c_uint64),
                 ("bvh_prim_count", C.c_uint64), ("nonfinite_values", C.c_uint64), ("primary_rays_culled", C.c_uint64), ("final_rays_skipped", C.c_uint64), ("bvh_fallback_lbvh", C.c_uint64),
-                ("gather_ms", C.c_double), ("pixels_dropped", C.c_uint64)]
+                ("gather_ms", C.c_double), ("pixels_dropped", C.c_uint64),
+                ("update_ms", C.c_double), ("bvh_sah_cost", C.c_double), ("bvh_last_update", C.c_uint64)]
 
 
 STATS_COUNTERS, STATS_KERNEL_TIMES = 1, 2
@@ -141,7 +142,7 @@ ABI_STRUCTS = [Camera, Shape, Instance, Light, Material, Texture, Image, SceneDe
                Outputs, PixelOutput, Stats]
 
 # every symbol include/rtcuda.h declares
-EXPORTED_SYMBOLS = ["rtcuda_init", "rtcuda_shutdown", "rtcuda_scene_upload", "rtcuda_scene_release", "rtcuda_release_cached_memory", "rtcuda_render",
+EXPORTED_SYMBOLS = ["rtcuda_init", "rtcuda_shutdown", "rtcuda_scene_upload", "rtcuda_scene_update", "rtcuda_scene_release", "rtcuda_release_cached_memory", "rtcuda_render",
                     "rtcuda_render_device", "rtcuda_render_samples_device", "rtcuda_render_samples_accumulate_device", "rtcuda_render_pixel", "rtcuda_get_stats", "rtcuda_last_error",
                     "rtcuda_abi_version", "rtcuda_abi_struct_sizes", "rtcuda_host_alloc", "rtcuda_host_free"]
 
@@ -172,6 +173,8 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.rtcuda_shutdown.restype = None
     lib.rtcuda_scene_upload.argtypes = [C.c_void_p, C.POINTER(SceneDesc), C.POINTER(C.c_void_p)]
     lib.rtcuda_scene_upload.restype = C.c_int
+    lib.rtcuda_scene_update.argtypes = [C.c_void_p, C.POINTER(SceneDesc)]
+    lib.rtcuda_scene_update.restype = C.c_int
     lib.rtcuda_scene_release.argtypes = [C.c_void_p]
     lib.rtcuda_scene_release.restype = None
     lib.rtcuda_host_alloc.argtypes = [C.c_size_t]

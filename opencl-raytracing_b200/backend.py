@@ -111,6 +111,15 @@ class CudaRenderer:
         except Exception:
             pass
 
+    def update(self, scene: Scene) -> None:
+        """Move the camera, the instance transforms and the lights of the uploaded scene to those of `scene`, which must have
+        the uploaded scene's topology (same shapes, instances -> shapes, light kinds, materials, textures, raster size and
+        camera kind; rtcuda_scene_update). The BVH is refitted (or rebuilt) on the device; no geometry is copied again, and
+        the next frame equals the frame of a fresh CudaRenderer(scene)."""
+        holder = scene.to_desc(own_arrays=True)   # zero-copy: the library reads no mesh array
+        _ffi.check(self.lib, self.lib.rtcuda_scene_update(self._scene, C.byref(holder.desc)), "rtcuda_scene_update")
+        self.scene = scene
+
     def render(self, settings: RaytracerSettings) -> RenderOutput:
         """raytracing_cpu::render: host planes, row-major [H,W,C]."""
         out = RenderOutput.allocate(self.width, self.height, AovFlags(settings.outputs), lib=self.lib)

@@ -396,6 +396,16 @@ struct rtcuda_scene {
     DevBuf<Prim> prims;
     DevBuf<ShadeRec> shade_recs;
     std::vector<rtcuda_light> host_lights;
+    // What rtcuda_scene_update compares a new description against: the camera and the instance rows as uploaded
+    rtcuda_camera host_camera{};
+    std::vector<Instance> host_instances;
+    std::vector<LightD> light_rows;
+    uint32_t shape_count = 0, material_count = 0, texture_count = 0, image_count = 0;
+    // Wide BVH levels (nodes per level, root first; level L + 1 is the contiguous node range the collapse of level L
+    // allocated) and, from the first update on, every node's float box and SAH term (RefitCtx::node_box)
+    std::vector<uint32_t> level_counts;
+    DevBuf<float4> node_box;
+    double sah_built = 0.0;   // SAH cost of the tree as last built (0: not computed yet)
     // Multi-device scene: the per-GPU scenes (subs[r] belongs to ctx->subs[r]); the parent holds nothing else of the above.
     std::vector<rtcuda_scene*> subs;
     // ... and, in each sub-scene, what the exchange of owned pixels needs (multi_* functions below): the packed planes of this
@@ -652,6 +662,7 @@ void build_bvh(rtcuda_scene* s, const std::vector<Instance>& instances, uint32_t
     s->sc.prim_count = n_prims;
     s->sc.node_count = 0;
     if (n_prims == 0) {
+        s->level_counts.clear();
         s->nodes.alloc(1);
         s->prims.alloc(1);
         s->sc.scene_center[0] = s->sc.scene_center[1] = s->sc.scene_center[2] = 0.0f;
@@ -787,6 +798,8 @@ void build_bvh(rtcuda_scene* s, const std::vector<Instance>& instances, uint32_t
         n_levels += queued;
     }
     CK(cudaMemcpyAsync(h_counters, counters.p, sizeof h_counters, cudaMemcpyDeviceToHost, st));
+    s->level_counts.resize(n_levels);
+    CK(cudaMemcpyAsync(s->level_counts.data(), level_count.p, n_levels * 4, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     if (!use_lbvh && std::getenv("RTCUDA_TEST_PLOC_TOO_DEEP")) too_deep = true;   // test hook for the fallback below
     if (!too_deep) break;
@@ -979,6 +992,10 @@ void upload_scene(rtcuda_scene* s, const rtcuda_scene_desc* d, const GeoShare* s
         }
     }
     s->host_lights.assign(d->lights, d->lights + d->light_count);
+    s->host_camera = d->camera;
+    s->host_instances = instances;
+    s->light_rows = lights;
+    s->shape_count = d->shape_count; s->material_count = d->material_count; s->texture_count = d->texture_count; s->image_count = d->image_count;
     std::vector<MaterialD> materials(d->material_count);
     for (uint32_t i = 0; i < d->material_count; i++) {
         const rtcuda_material& a = d->materials[i];
@@ -1538,6 +1555,184 @@ void render_pixel(rtcuda_scene* s, const rtcuda_settings* settings, uint32_t x, 
 
 
 // ---------------------------------------------------------------------------------------------------
+// scene update: camera, instance transforms and lights of an uploaded scene, in place
+// ---------------------------------------------------------------------------------------------------
+// The description must have the uploaded scene's topology; only what update_scene reads is checked, and all of it before any
+// device work, so a refused update leaves the scene as it was.
+void validate_update(const rtcuda_scene* s, const rtcuda_scene_desc* d) {
+    REQUIRE(d->abi_version == RTCUDA_ABI_VERSION, "scene_desc.abi_version mismatch");
+    REQUIRE(d->camera.raster_width == s->host_camera.raster_width && d->camera.raster_height == s->host_camera.raster_height,
+            "update: the raster size differs from the uploaded scene's");
+    REQUIRE(d->camera.kind == s->host_camera.kind, "update: the camera kind differs from the uploaded scene's");
+    REQUIRE(d->shape_count == s->shape_count && d->instance_count == s->host_instances.size() && d->light_count == s->host_lights.size() &&
+                d->material_count == s->material_count && d->texture_count == s->texture_count && d->image_count == s->image_count,
+            "update: the shape / instance / light / material / texture / image counts differ from the uploaded scene's");
+    REQUIRE(d->instance_count == 0 || d->instances, "update: instances is NULL");
+    REQUIRE(d->light_count == 0 || d->lights, "update: lights is NULL");
+    for (uint32_t i = 0; i < d->instance_count; i++)
+        REQUIRE(d->instances[i].shape == s->host_instances[i].shape, "update: an instance refers to another shape than the uploaded one");
+    for (uint32_t i = 0; i < d->light_count; i++)
+        REQUIRE(d->lights[i].kind == s->host_lights[i].kind && d->lights[i].shape == s->host_lights[i].shape,
+                "update: a light's kind or shape differs from the uploaded one");
+}
+
+// Node pass over every level, deepest first, then the deterministic SAH sum; returns the cost (RefitCtx::node_box)
+double refit_nodes(rtcuda_scene* s, RefitCtx& r, bool write_nodes) {
+    cudaStream_t st = s->ctx->stream;
+    r.write_nodes = write_nodes ? 1u : 0u;
+    std::vector<uint32_t> first(s->level_counts.size());
+    uint32_t n_nodes = 0;
+    for (size_t L = 0; L < s->level_counts.size(); L++) { first[L] = n_nodes; n_nodes += s->level_counts[L]; }
+    for (size_t L = s->level_counts.size(); L-- > 0;) launch_refit_nodes(st, r, first[L], s->level_counts[L], s->lc);
+    DevBuf<double> partial;
+    partial.alloc(SAH_BLOCKS);
+    launch_sah_partial(st, r.node_box, n_nodes, partial.p, s->lc);
+    double h_partial[SAH_BLOCKS];
+    float4 root[2];
+    CK(cudaMemcpyAsync(h_partial, partial.p, sizeof h_partial, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(root, r.node_box, sizeof root, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    double children = 0.0;
+    for (uint32_t b = 0; b < SAH_BLOCKS; b++) children += h_partial[b];
+    return sah_cost(root, children);
+}
+
+void update_scene(rtcuda_scene* s, const rtcuda_scene_desc* d) {
+    cudaStream_t st = s->ctx->stream;
+    Trace tr("update", (int)s->ctx->bs.tile_rank);
+    const bool cam_changed = std::memcmp(&d->camera, &s->host_camera, sizeof d->camera) != 0;
+    bool lights_changed = false, moved = false;
+    for (uint32_t i = 0; i < d->light_count; i++) {
+        const rtcuda_light& a = d->lights[i];
+        const rtcuda_light& h = s->host_lights[i];
+        lights_changed |= std::memcmp(a.position_or_direction, h.position_or_direction, sizeof a.position_or_direction) != 0 ||
+                          std::memcmp(a.intensity_or_radiance, h.intensity_or_radiance, sizeof a.intensity_or_radiance) != 0 ||
+                          std::memcmp(&a.light_to_world, &h.light_to_world, sizeof a.light_to_world) != 0;
+    }
+    std::vector<uint8_t> row_moved(d->instance_count, 0);
+    for (uint32_t i = 0; i < d->instance_count; i++) {
+        const Instance& h = s->host_instances[i];
+        const M4 f = to_m4(d->instances[i].object_to_world.forward), v = to_m4(d->instances[i].object_to_world.inverse);
+        row_moved[i] = std::memcmp(&f, &h.o2w, sizeof f) != 0 || std::memcmp(&v, &h.w2o, sizeof v) != 0;
+        moved |= row_moved[i] != 0;
+    }
+    const uint32_t n_prims = (uint32_t)s->stats.bvh_prim_count;
+    const bool have_tree = n_prims != 0;
+    if (have_tree && !RT_FIXED_SLOTS) throw RtError{RTCUDA_ERR_UNSUPPORTED, "scene updates need the fixed-slot primitive layout (RT_FIXED_SLOTS=1)"};
+    cudaEvent_t e0, e1;
+    CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
+    CK(cudaEventRecord(e0, st));
+
+    RefitCtx r{};
+    r.instances = s->instances.p; r.vertices = s->vertices.p; r.tris = s->tris.p;
+    r.prims = s->prims.p; r.prim_slots = s->sc.prim_count; r.nodes = s->nodes.p;
+    // the cost of the tree as built, from the unchanged primitives (first update of the scene; after a rebuild, below)
+    if (have_tree && s->sah_built == 0.0) {
+        s->node_box.alloc(2 * (size_t)s->sc.node_count);
+        r.node_box = s->node_box.p;
+        s->sah_built = refit_nodes(s, r, false);
+        s->stats.bvh_sah_cost = s->sah_built;
+    }
+    r.node_box = s->node_box.p;
+    tr.mark("baseline");
+
+    // instance rows: runs of moved rows, one copy each
+    for (uint32_t i = 0; i < d->instance_count;) {
+        if (!row_moved[i]) { i++; continue; }
+        uint32_t j = i;
+        for (; j < d->instance_count && row_moved[j]; j++) {
+            s->host_instances[j].o2w = to_m4(d->instances[j].object_to_world.forward);
+            s->host_instances[j].w2o = to_m4(d->instances[j].object_to_world.inverse);
+        }
+        CK(cudaMemcpyAsync(s->instances.p + i, s->host_instances.data() + i, (j - i) * sizeof(Instance), cudaMemcpyHostToDevice, st));
+        i = j;
+    }
+    if (lights_changed) {
+        for (uint32_t i = 0; i < d->light_count; i++) {
+            const rtcuda_light& a = d->lights[i];
+            LightD& b = s->light_rows[i];
+            std::memcpy(b.a, a.position_or_direction, sizeof b.a);
+            std::memcpy(b.b, a.intensity_or_radiance, sizeof b.b);
+            b.light_to_world = to_m4(a.light_to_world);
+            s->host_lights[i] = a;
+        }
+        CK(cudaMemcpyAsync(s->lights.p, s->light_rows.data(), s->light_rows.size() * sizeof(LightD), cudaMemcpyHostToDevice, st));
+        s->sc.light0 = s->light_rows[0];
+    }
+    if (cam_changed) {
+        CameraD& cam = s->sc.camera;
+        cam.near_clip = d->camera.near_clip; cam.far_clip = d->camera.far_clip;
+        cam.aperture_radius = d->camera.aperture_radius; cam.focal_distance = d->camera.focal_distance;
+        cam.raster_to_camera = to_m4(d->camera.raster_to_camera.forward);
+        cam.camera_to_world = to_m4(d->camera.camera_to_world.forward);
+        s->host_camera = d->camera;
+    }
+
+    uint32_t last = cam_changed || lights_changed ? 1u : 0u;
+    if (moved && have_tree) {
+        DevBuf<uint32_t> bounds_keys;
+        bounds_keys.alloc(6);
+        const uint32_t init_keys[6] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u};
+        CK(cudaMemcpyAsync(bounds_keys.p, init_keys, sizeof init_keys, cudaMemcpyHostToDevice, st));
+        r.bounds_keys = bounds_keys.p;
+        launch_refit_prims(st, r, s->lc);
+        const double sah_refit = refit_nodes(s, r, true);
+        tr.mark("refit");
+        // RTCUDA_TEST_REFIT_MAX_GROWTH: test / measurement hook that replaces the rule's factor (scripts/update_bench.py keeps
+        // every refit with a huge value, to measure what a refit costs where the rule would rebuild)
+        const char* growth = std::getenv("RTCUDA_TEST_REFIT_MAX_GROWTH");
+        if (refit_needs_rebuild(sah_refit, s->sah_built, growth ? std::atof(growth) : REFIT_MAX_GROWTH)) {
+            // from the resident geometry: the instance table on the device is current
+            build_bvh(s, s->host_instances, n_prims);
+            s->sc.nodes = s->nodes.p;
+            s->sc.prims = s->prims.p;
+            s->shade_recs.alloc(s->sc.prim_count);
+            launch_shade_recs(st, s->sc, s->shade_recs.p, s->lc);
+            s->sc.shade_recs = s->shade_recs.p;
+            s->node_box.alloc(2 * (size_t)s->sc.node_count);
+            r.prims = s->prims.p; r.prim_slots = s->sc.prim_count; r.nodes = s->nodes.p; r.node_box = s->node_box.p;
+            s->sah_built = refit_nodes(s, r, false);
+            s->stats.bvh_sah_cost = s->sah_built;
+            last = 3;
+            tr.mark("rebuild");
+        } else {
+            // scene centre, radius and culling bounds from the refitted primitives, exactly as build_bvh derives them
+            uint32_t hk[6];
+            CK(cudaMemcpyAsync(hk, bounds_keys.p, sizeof hk, cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            const V3 mn = mk3(key_float(hk[0]), key_float(hk[1]), key_float(hk[2])), mx = mk3(key_float(hk[3]), key_float(hk[4]), key_float(hk[5]));
+            const V3 c = (mx + mn) / 2.0f;
+            s->sc.scene_center[0] = c.x; s->sc.scene_center[1] = c.y; s->sc.scene_center[2] = c.z;
+            s->sc.scene_radius = n_prims == 1 ? INFINITY : length(mx - c);
+            set_scene_bounds(s->sc, mn, mx, true);
+            s->stats.bvh_sah_cost = sah_refit;
+            last = 2;
+        }
+    } else if (moved) last = 1;   // instances without primitives: nothing in the tree moves
+    if (last) {
+        // Everything derived from the camera, the lights or the bounds: the captured frame graph (its launches hold the old
+        // kernel parameters, and its key sees neither the camera nor the scene constants), the pixel lists and the tile table
+        // (the culling rectangle of build_pixel_list is the projected scene bounds).
+        reset_spans(s);
+        s->frame_key.clear();
+        s->seen_key.clear();
+        s->pixel_list.release();
+        s->beauty_list_buf.release();
+        s->beauty_list = nullptr;
+        s->n_my_pixels = s->n_beauty_pixels = 0;
+        s->host_tiles.clear();
+        s->tiles.release();
+    }
+    CK(cudaEventRecord(e1, st));
+    CK(cudaStreamSynchronize(st));
+    float ms = 0;
+    CK(cudaEventElapsedTime(&ms, e0, e1));
+    cudaEventDestroy(e0); cudaEventDestroy(e1);
+    s->stats.update_ms = ms;
+    s->stats.bvh_last_update = last;
+}
+
+// ---------------------------------------------------------------------------------------------------
 // multi-device contexts (backend_settings.num_devices > 1): the scene replicated on every GPU, tiles dealt round-robin,
 // one host thread per GPU per call — the in-process analogue of the CPU backend's worker pool (lib.rs:706-805)
 // ---------------------------------------------------------------------------------------------------
@@ -1590,6 +1785,21 @@ void multi_upload(rtcuda_ctx* ctx, const rtcuda_scene_desc* desc, rtcuda_scene* 
             throw;
         }
     });
+}
+
+// Validated once against rank 0's copies (every rank holds the same), then every GPU updates its replica on its own thread. Rank 0's
+// copies of the other ranks' tile tables go with their pixel lists.
+void multi_update(rtcuda_scene* parent, const rtcuda_scene_desc* desc) {
+    validate_update(parent->subs[0], desc);
+    for_each_device(parent->subs.size(), [&](size_t r) {
+        enter(parent->subs[r]);
+        update_scene(parent->subs[r], desc);
+    });
+    rtcuda_scene* first = parent->subs[0];
+    if (first->stats.bvh_last_update) {
+        enter(first);
+        for (TileRec*& q : first->peer_list) { if (q) cudaFree(q); q = nullptr; }
+    }
 }
 
 void multi_release(rtcuda_scene* parent) {
@@ -1798,7 +2008,12 @@ rtcuda_stats multi_stats(const rtcuda_scene* parent) {
         t.extend_ms = std::max(t.extend_ms, a.extend_ms); t.shade_ms = std::max(t.shade_ms, a.shade_ms); t.shadow_ms = std::max(t.shadow_ms, a.shadow_ms);
         t.other_ms = std::max(t.other_ms, a.other_ms); t.gather_ms = std::max(t.gather_ms, a.gather_ms);
         t.pixels_dropped += a.pixels_dropped;
-        if (first) { t.bvh_node_count = a.bvh_node_count; t.bvh_prim_count = a.bvh_prim_count; first = false; }
+        t.update_ms = std::max(t.update_ms, a.update_ms);
+        if (first) {
+            t.bvh_node_count = a.bvh_node_count; t.bvh_prim_count = a.bvh_prim_count;
+            t.bvh_sah_cost = a.bvh_sah_cost; t.bvh_last_update = a.bvh_last_update;   // (the same on every GPU: same data, same decision)
+            first = false;
+        }
     }
     return t;
 }
@@ -1931,6 +2146,17 @@ RTCUDA_API rtcuda_status rtcuda_scene_upload(rtcuda_ctx* ctx, const rtcuda_scene
         tls_stream = ctx->stream;
         upload_scene(s.get(), desc);
         *out_scene = s.release();
+    });
+}
+
+RTCUDA_API rtcuda_status rtcuda_scene_update(rtcuda_scene* scene, const rtcuda_scene_desc* desc) {
+    return guarded([&] {
+        REQUIRE(scene && desc, "null argument");
+        if (!scene->subs.empty()) { multi_update(scene, desc); return; }
+        validate_update(scene, desc);
+        CK(cudaSetDevice(scene->ctx->device));
+        tls_stream = scene->ctx->stream;
+        update_scene(scene, desc);
     });
 }
 

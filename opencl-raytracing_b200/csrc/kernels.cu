@@ -566,6 +566,59 @@ void launch_collapse(cudaStream_t st, const BuildCtx& b, uint32_t bound, uint32_
     lc.launches += 2;
 }
 
+// Refit (rtcuda_scene_update). One thread per primitive slot; the bounds are min / max of order-preserving keys, exact in any
+// order, so a warp reduces its keys before one lane does the six atomics (one atomic per slot on six addresses serialises).
+__global__ void __launch_bounds__(BLOCK) k_refit_prims(RefitCtx r) {
+    const uint32_t i = blockIdx.x * BLOCK + threadIdx.x;
+    V3 lo, hi;
+    const bool filled = i < r.prim_slots && refit_prims_body(i, r, lo, hi);
+    uint32_t k[6] = {0xffffffffu, 0xffffffffu, 0xffffffffu, 0u, 0u, 0u};
+    if (filled) {
+        k[0] = float_key(lo.x); k[1] = float_key(lo.y); k[2] = float_key(lo.z);
+        k[3] = float_key(hi.x); k[4] = float_key(hi.y); k[5] = float_key(hi.z);
+    }
+    if (!__any_sync(0xffffffffu, filled)) return;
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+        k[a] = __reduce_min_sync(0xffffffffu, k[a]);
+        k[3 + a] = __reduce_max_sync(0xffffffffu, k[3 + a]);
+    }
+    if ((threadIdx.x & 31u) == 0) {
+#pragma unroll
+        for (int a = 0; a < 3; a++) { atomicMin(&r.bounds_keys[a], k[a]); atomicMax(&r.bounds_keys[3 + a], k[3 + a]); }
+    }
+}
+__global__ void __launch_bounds__(128) k_refit_nodes(RefitCtx r, uint32_t first, uint32_t count) {
+    const uint32_t i = blockIdx.x * 128 + threadIdx.x;
+    if (i < count) refit_nodes_body(first + i, r);
+}
+// per-block sums of the nodes' SAH terms (node_box[2i].w), each block over a fixed strided subset in a fixed order (the host adds
+// the SAH_BLOCKS partials in block order): the same figure on every run and every GPU
+__global__ void __launch_bounds__(256) k_sah_partial(const float4* node_box, uint32_t n, double* partial) {
+    __shared__ double s[256];
+    double v = 0.0;
+    for (uint32_t i = blockIdx.x * 256 + threadIdx.x; i < n; i += SAH_BLOCKS * 256) v += (double)node_box[2 * (size_t)i].w;
+    s[threadIdx.x] = v;
+    __syncthreads();
+    for (uint32_t o = 128; o > 0; o >>= 1) {
+        if (threadIdx.x < o) s[threadIdx.x] += s[threadIdx.x + o];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) partial[blockIdx.x] = s[0];
+}
+void launch_refit_prims(cudaStream_t st, const RefitCtx& r, LaunchCounter& lc) {
+    k_refit_prims<<<grid_for(r.prim_slots), BLOCK, 0, st>>>(r);
+    lc.launches++;
+}
+void launch_refit_nodes(cudaStream_t st, const RefitCtx& r, uint32_t first, uint32_t count, LaunchCounter& lc) {
+    k_refit_nodes<<<grid_for(count, 128), 128, 0, st>>>(r, first, count);
+    lc.launches++;
+}
+void launch_sah_partial(cudaStream_t st, const float4* node_box, uint32_t n, double* partial, LaunchCounter& lc) {
+    k_sah_partial<<<SAH_BLOCKS, 256, 0, st>>>(node_box, n, partial);
+    lc.launches++;
+}
+
 void launch_ploc_init(cudaStream_t st, const BuildCtx& b, LaunchCounter& lc) { k_ploc_init<<<grid_for(b.n), BLOCK, 0, st>>>(b); lc.launches++; }
 size_t ploc_scan_temp_bytes(uint32_t n) {
     size_t bytes = 0;

@@ -51,6 +51,12 @@ void launch_ploc_tail(cudaStream_t st, const BuildCtx& b, const uint32_t* state,
 void launch_ploc_round(cudaStream_t st, const BuildCtx& b, uint32_t bound, const uint32_t* state, uint32_t* state_next, void* scan_temp,
                        size_t scan_temp_bytes, LaunchCounter& lc);
 
+// refit of the wide BVH (rtcuda_scene_update): primitive slots, then one launch per wide level (deepest first), then the SAH terms
+void launch_refit_prims(cudaStream_t st, const RefitCtx& r, LaunchCounter& lc);
+void launch_refit_nodes(cudaStream_t st, const RefitCtx& r, uint32_t first, uint32_t count, LaunchCounter& lc);
+constexpr uint32_t SAH_BLOCKS = 256;   // partial sums launch_sah_partial writes (doubles)
+void launch_sah_partial(cudaStream_t st, const float4* node_box, uint32_t n, double* partial, LaunchCounter& lc);
+
 // emitter triangle table (rt_scene.h LightTri)
 void launch_check_indices(cudaStream_t st, const uint32_t* idx, size_t n, uint32_t vertex_count, uint32_t* bad, LaunchCounter& lc);
 void launch_light_tris(cudaStream_t st, const ShapeD* shapes, uint32_t shape, uint32_t tri_count, const float* vertices, const uint32_t* tris,

@@ -85,37 +85,47 @@ RT_HD uint32_t instance_of_prim(const BuildCtx& b, uint32_t i) {
     return lo;
 }
 
-RT_HD void prim_setup_body(uint32_t i, const BuildCtx& b) {
-    uint32_t g = instance_of_prim(b, i);
-    const Instance& inst = b.instances[g];
-    uint32_t local = i - inst.prim_base;
-    V3 lo, hi;
-    Prim p;
+// The 8 transformed corners of a sphere instance's object box (aabb.rs:81-95): its world box in the build and in the refit.
+RT_HD void sphere_box(const Instance& inst, V3& lo, V3& hi) {
+    V3 c = mk3(inst.center[0], inst.center[1], inst.center[2]);
+    V3 r = mk3(inst.radius);
+    V3 mn = c - r, mx = c + r;
+    lo = mk3(RT_INF, RT_INF, RT_INF);
+    hi = mk3(-RT_INF, -RT_INF, -RT_INF);
+    for (int k = 0; k < 8; k++) {
+        V3 q = apply_point(inst.o2w, mk3((k & 4) ? mx.x : mn.x, (k & 2) ? mx.y : mn.y, (k & 1) ? mx.z : mn.z));
+        lo = vmin(lo, q);
+        hi = vmax(hi, q);
+    }
+}
+
+// Primitive `local` of instance g in world space and its world box: the one definition the build (prim_setup_body) and the
+// refit (refit_prims_body) share, so a refit with unchanged transforms writes the bits a fresh build writes.
+RT_HD void world_prim(const Instance& inst, uint32_t g, uint32_t local, const float* vertices, const uint32_t* tris, Prim& p, V3& lo, V3& hi) {
     if (inst.kind == 0) {
-        const uint32_t* t = b.tris + 3 * (size_t)(inst.tri_offset + local);
-        V3 v0 = apply_point(inst.o2w, load3(b.vertices, inst.vertex_offset + t[0]));
-        V3 v1 = apply_point(inst.o2w, load3(b.vertices, inst.vertex_offset + t[1]));
-        V3 v2 = apply_point(inst.o2w, load3(b.vertices, inst.vertex_offset + t[2]));
+        const uint32_t* t = tris + 3 * (size_t)(inst.tri_offset + local);
+        V3 v0 = apply_point(inst.o2w, load3(vertices, inst.vertex_offset + t[0]));
+        V3 v1 = apply_point(inst.o2w, load3(vertices, inst.vertex_offset + t[1]));
+        V3 v2 = apply_point(inst.o2w, load3(vertices, inst.vertex_offset + t[2]));
         lo = vmin(v0, vmin(v1, v2));
         hi = vmax(v0, vmax(v1, v2));
         p.a = make_float4(v0.x, v0.y, v0.z, u2f(g));
         p.b = make_float4(v1.x, v1.y, v1.z, u2f(local));
         p.c = make_float4(v2.x, v2.y, v2.z, u2f(0u));
     } else {
-        V3 c = mk3(inst.center[0], inst.center[1], inst.center[2]);
-        V3 r = mk3(inst.radius);
-        V3 mn = c - r, mx = c + r;
-        lo = mk3(RT_INF, RT_INF, RT_INF);
-        hi = mk3(-RT_INF, -RT_INF, -RT_INF);
-        for (int k = 0; k < 8; k++) {  // aabb.rs:81-95
-            V3 q = apply_point(inst.o2w, mk3((k & 4) ? mx.x : mn.x, (k & 2) ? mx.y : mn.y, (k & 1) ? mx.z : mn.z));
-            lo = vmin(lo, q);
-            hi = vmax(hi, q);
-        }
-        p.a = make_float4(c.x, c.y, c.z, u2f(g));
+        sphere_box(inst, lo, hi);
+        p.a = make_float4(inst.center[0], inst.center[1], inst.center[2], u2f(g));
         p.b = make_float4(inst.radius, 0.0f, 0.0f, u2f(0u));
         p.c = make_float4(0.0f, 0.0f, 0.0f, u2f(1u));
     }
+}
+
+RT_HD void prim_setup_body(uint32_t i, const BuildCtx& b) {
+    uint32_t g = instance_of_prim(b, i);
+    const Instance& inst = b.instances[g];
+    V3 lo, hi;
+    Prim p;
+    world_prim(inst, g, i - inst.prim_base, b.vertices, b.tris, p, lo, hi);
     b.prims_unsorted[i] = p;
     b.aabb_lo[i] = make_float4(lo.x, lo.y, lo.z, 0.0f);
     b.aabb_hi[i] = make_float4(hi.x, hi.y, hi.z, 0.0f);
@@ -280,6 +290,53 @@ RT_HD void ploc_merge_body(uint32_t i, const BuildCtx& b) {
     if (i == b.m - 1) { b.ploc_out[0] = pos + 1u; b.ploc_out[1] = rank + (mutual ? 1u : 0u); }
 }
 
+// ---- quantised node planes (shared by the collapse and the refit) ------------------------------------------
+// exponents: smallest power of two with lo + 255 * 2^e >= hi
+RT_HD void node_exponents(V3 lo, V3 hi, uint32_t ebits[3]) {
+    const float ext[3] = {hi.x - lo.x, hi.y - lo.y, hi.z - lo.z};
+    const float lov[3] = {lo.x, lo.y, lo.z}, hiv[3] = {hi.x, hi.y, hi.z};
+    for (int a = 0; a < 3; a++) {
+        int e = 1;  // biased exponent
+        if (ext[a] > 0.0f) {
+            int ex;
+            frexpf(ext[a] / 255.0f, &ex);  // ext/255 = m * 2^ex, m in [0.5, 1)
+            e = ex + 127;
+            if (e < 1) e = 1;
+            if (e > 238) e = 238;  // rt_traverse.h folds 2^15 into the scale: e + 15 must stay a finite exponent
+            while (e < 238 && lov[a] + 255.0f * u2f((uint32_t)e << 23) < hiv[a]) e++;
+        }
+        ebits[a] = (uint32_t)e;
+    }
+}
+
+// the conservative 8-bit planes of child box [cl, ch] in slot s of a node with origin `lo`
+RT_HD void quantize_child(const uint32_t ebits[3], V3 lo, V3 clo, V3 chi, int s, uint32_t q[6][8]) {
+    const float lov[3] = {lo.x, lo.y, lo.z};
+    const float cl[3] = {clo.x, clo.y, clo.z}, chh[3] = {chi.x, chi.y, chi.z};
+    for (int a = 0; a < 3; a++) {
+        const float scale = u2f(ebits[a] << 23);
+        float ql = floorf((cl[a] - lov[a]) / scale);
+        float qh = ceilf((chh[a] - lov[a]) / scale);
+        ql = fminf(fmaxf(ql, 0.0f), 255.0f);
+        qh = fminf(fmaxf(qh, 0.0f), 255.0f);
+        while (ql > 0.0f && lov[a] + ql * scale > cl[a]) ql -= 1.0f;
+        while (qh < 255.0f && lov[a] + qh * scale < chh[a]) qh += 1.0f;
+        if (qh <= ql) { if (qh < 255.0f) qh = ql + 1.0f; else ql = qh - 1.0f; }  // never a zero-thickness slab
+        q[a][s] = (uint32_t)ql;
+        q[3 + a][s] = (uint32_t)qh;
+    }
+}
+
+RT_HD uint32_t pack4(const uint32_t* v) { return v[0] | (v[1] << 8) | (v[2] << 16) | (v[3] << 24); }
+
+// n0 and the plane words n2..n4 of a node (n1 is the caller's)
+RT_HD void pack_node_planes(Node8& nd8, V3 lo, const uint32_t ebits[3], uint32_t imask, uint32_t q[6][8]) {
+    nd8.n0 = make_float4(lo.x, lo.y, lo.z, u2f(ebits[0] | (ebits[1] << 8) | (ebits[2] << 16) | (imask << 24)));
+    nd8.n2 = make_float4(u2f(pack4(q[0])), u2f(pack4(q[0] + 4)), u2f(pack4(q[1])), u2f(pack4(q[1] + 4)));
+    nd8.n3 = make_float4(u2f(pack4(q[2])), u2f(pack4(q[2] + 4)), u2f(pack4(q[3])), u2f(pack4(q[3] + 4)));
+    nd8.n4 = make_float4(u2f(pack4(q[4])), u2f(pack4(q[4] + 4)), u2f(pack4(q[5])), u2f(pack4(q[5] + 4)));
+}
+
 // One wide node per work item: gather up to 8 children by repeatedly opening the binary child with
 // the largest surface area, order them into octant slots, quantise, emit child work items.
 RT_HD void collapse_body(uint32_t item_idx, const BuildCtx& b) {
@@ -356,24 +413,8 @@ RT_HD void collapse_body(uint32_t item_idx, const BuildCtx& b) {
         child_in[bs] = bc;
     }
 
-    // exponents: smallest power of two with lo + 255 * 2^e >= hi
     uint32_t ebits[3];
-    float scale[3];
-    const float ext[3] = {hi.x - lo.x, hi.y - lo.y, hi.z - lo.z};
-    const float lov[3] = {lo.x, lo.y, lo.z}, hiv[3] = {hi.x, hi.y, hi.z};
-    for (int a = 0; a < 3; a++) {
-        int e = 1;  // biased exponent
-        if (ext[a] > 0.0f) {
-            int ex;
-            frexpf(ext[a] / 255.0f, &ex);  // ext/255 = m * 2^ex, m in [0.5, 1)
-            e = ex + 127;
-            if (e < 1) e = 1;
-            if (e > 238) e = 238;  // rt_traverse.h folds 2^15 into the scale: e + 15 must stay a finite exponent
-            while (e < 238 && lov[a] + 255.0f * u2f((uint32_t)e << 23) < hiv[a]) e++;
-        }
-        ebits[a] = (uint32_t)e;
-        scale[a] = u2f((uint32_t)e << 23);
-    }
+    node_exponents(lo, hi, ebits);
 
     uint32_t n_internal = 0, n_leaf_prims = 0;
     for (int s = 0; s < 8; s++) {
@@ -406,18 +447,7 @@ RT_HD void collapse_body(uint32_t item_idx, const BuildCtx& b) {
         if (c < 0) continue;
         uint32_t nd = ch[c];
         uint32_t cnt = b.count[nd];
-        const float cl[3] = {clo[c].x, clo[c].y, clo[c].z}, chh[3] = {chi[c].x, chi[c].y, chi[c].z};
-        for (int a = 0; a < 3; a++) {
-            float ql = floorf((cl[a] - lov[a]) / scale[a]);
-            float qh = ceilf((chh[a] - lov[a]) / scale[a]);
-            ql = fminf(fmaxf(ql, 0.0f), 255.0f);
-            qh = fminf(fmaxf(qh, 0.0f), 255.0f);
-            while (ql > 0.0f && lov[a] + ql * scale[a] > cl[a]) ql -= 1.0f;
-            while (qh < 255.0f && lov[a] + qh * scale[a] < chh[a]) qh += 1.0f;
-            if (qh <= ql) { if (qh < 255.0f) qh = ql + 1.0f; else ql = qh - 1.0f; }  // never a zero-thickness slab
-            q[a][s] = (uint32_t)ql;
-            q[3 + a][s] = (uint32_t)qh;
-        }
+        quantize_child(ebits, lo, clo[c], chi[c], s, q);
         if (cnt <= LEAF_MAX) {
 #if RT_FIXED_SLOTS
             k_prim = 3u * (uint32_t)s;
@@ -447,18 +477,124 @@ RT_HD void collapse_body(uint32_t item_idx, const BuildCtx& b) {
         }
     }
 
-    auto pack4 = [](const uint32_t* v) { return v[0] | (v[1] << 8) | (v[2] << 16) | (v[3] << 24); };
     Node8 nd8;
-    nd8.n0 = make_float4(lo.x, lo.y, lo.z, u2f(ebits[0] | (ebits[1] << 8) | (ebits[2] << 16) | (imask << 24)));
 #if RT_FIXED_SLOTS
     nd8.n1 = make_float4(u2f(child_base), u2f(prim_base), u2f(valid | (imask << 24)), u2f(0u));
 #else
     nd8.n1 = make_float4(u2f(child_base), u2f(prim_base), u2f(pack4(meta)), u2f(pack4(meta + 4)));
 #endif
-    nd8.n2 = make_float4(u2f(pack4(q[0])), u2f(pack4(q[0] + 4)), u2f(pack4(q[1])), u2f(pack4(q[1] + 4)));
-    nd8.n3 = make_float4(u2f(pack4(q[2])), u2f(pack4(q[2] + 4)), u2f(pack4(q[3])), u2f(pack4(q[3] + 4)));
-    nd8.n4 = make_float4(u2f(pack4(q[4])), u2f(pack4(q[4] + 4)), u2f(pack4(q[5])), u2f(pack4(q[5] + 4)));
+    pack_node_planes(nd8, lo, ebits, imask, q);
     b.nodes[it.wnode] = nd8;
+}
+
+// ---- refit (rtcuda_scene_update) ------------------------------------------------------------------------------
+// Moving instances keeps the tree: every filled primitive slot records its (geom, prim, kind), so it is recomputed in place
+// from the updated Instance (refit_prims_body), and the wide nodes are re-fitted bottom-up, one launch per level, deepest
+// first (refit_nodes_body). Child slots, child_base / prim_base / valid and the primitive order stay as they are; the node
+// frame, exponents and planes are recomputed by the code the collapse uses. Traversal results do not depend on the tree
+// (closest t, ties to the larger (geom, prim); conservative boxes, exact primitive tests), so a refitted tree renders the
+// frame a fresh build of the same transforms renders.
+struct RefitCtx {
+    const Instance* instances;
+    const float* vertices;
+    const uint32_t* tris;
+    Prim* prims;
+    uint32_t prim_slots;
+    uint32_t* bounds_keys;      // 6 x u32 float_key: min xyz, max xyz (initialised by the caller)
+    Node8* nodes;
+    // 2 per node: (lo.xyz | SAH term of the node's children), (hi.xyz | -): the float box the parent's refit reads
+    float4* node_box;
+    uint32_t write_nodes;       // 0: only node_box (the cost of the tree as it is, without touching a node)
+};
+
+// Recomputes slot i; false for a hole. lo / hi: the primitive's world box (for the bounds reduction).
+RT_HD bool refit_prims_body(uint32_t i, const RefitCtx& r, V3& lo, V3& hi) {
+    const Prim old = r.prims[i];
+    if (f2u(old.c.w) == PRIM_HOLE) return false;
+    const uint32_t g = f2u(old.a.w);
+    Prim p;
+    world_prim(r.instances[g], g, f2u(old.b.w), r.vertices, r.tris, p, lo, hi);
+    r.prims[i] = p;
+    return true;
+}
+
+// World box of a filled slot: the triangle's vertices as stored, or the sphere's transformed object box
+RT_HD void prim_world_box(const Prim& p, const Instance* instances, V3& lo, V3& hi) {
+    if (f2u(p.c.w) == 0u) {
+        const V3 v0 = xyz(p.a), v1 = xyz(p.b), v2 = xyz(p.c);
+        lo = vmin(v0, vmin(v1, v2));
+        hi = vmax(v0, vmax(v1, v2));
+    } else sphere_box(instances[f2u(p.a.w)], lo, hi);
+}
+
+// Node i of a level whose children (a deeper level) are refitted already.
+RT_HD void refit_nodes_body(uint32_t i, const RefitCtx& r) {
+    Node8 nd = r.nodes[i];
+    const uint32_t child_base = f2u(nd.n1.x), prim_base = f2u(nd.n1.y), valid = f2u(nd.n1.z);
+    const uint32_t imask = valid >> 24;
+    V3 clo[8], chi[8];
+    V3 lo = mk3(RT_INF, RT_INF, RT_INF), hi = mk3(-RT_INF, -RT_INF, -RT_INF);
+    float sah = 0.0f;
+    uint32_t k_internal = 0, present = 0;
+#pragma unroll
+    for (int s = 0; s < 8; s++) {
+        if (imask & (1u << s)) {
+            const uint32_t c = child_base + k_internal++;
+            clo[s] = xyz(r.node_box[2 * (size_t)c]);
+            chi[s] = xyz(r.node_box[2 * (size_t)c + 1]);
+            sah += half_area(clo[s], chi[s]);
+        } else {
+            const uint32_t bits = (valid >> (3 * s)) & 7u;
+            if (!bits) continue;
+            clo[s] = mk3(RT_INF, RT_INF, RT_INF);
+            chi[s] = mk3(-RT_INF, -RT_INF, -RT_INF);
+            uint32_t cnt = 0;
+#pragma unroll
+            for (uint32_t k = 0; k < LEAF_MAX; k++) {
+                if (!(bits & (1u << k))) continue;
+                V3 plo, phi;
+                prim_world_box(r.prims[prim_base + 3u * (uint32_t)s + k], r.instances, plo, phi);
+                clo[s] = vmin(clo[s], plo);
+                chi[s] = vmax(chi[s], phi);
+                cnt++;
+            }
+            sah += half_area(clo[s], chi[s]) * (float)cnt;
+        }
+        present |= 1u << s;
+        lo = vmin(lo, clo[s]);
+        hi = vmax(hi, chi[s]);
+    }
+    r.node_box[2 * (size_t)i] = make_float4(lo.x, lo.y, lo.z, sah);
+    r.node_box[2 * (size_t)i + 1] = make_float4(hi.x, hi.y, hi.z, 0.0f);
+    if (!r.write_nodes) return;
+    uint32_t ebits[3], q[6][8];
+    node_exponents(lo, hi, ebits);
+#pragma unroll
+    for (int s = 0; s < 8; s++) {
+        for (int a = 0; a < 6; a++) q[a][s] = 0;
+        if (present & (1u << s)) quantize_child(ebits, lo, clo[s], chi[s], s, q);
+    }
+    pack_node_planes(nd, lo, ebits, imask, q);
+    r.nodes[i] = nd;
+}
+
+// SAH cost of the wide tree from the node boxes (C_node = C_prim = 1, A = half the surface area, a factor that cancels):
+// (A(root) + sum over inner children of A + sum over leaf children of A * primitives) / A(root).
+// `partial`: per-node terms summed in a fixed order (kernels.cu k_sah_partial), so every GPU gets the same figure.
+RT_HD double sah_cost(const float4* root_box, double children) {
+    const double a = half_area(xyz(root_box[0]), xyz(root_box[1]));
+    return a > 0.0 ? (a + children) / a : 0.0;
+}
+
+// Refit or rebuild: a refit whose SAH cost grew by more than this factor over the cost of the tree as last built is replaced
+// by a fresh build from the resident geometry. B200 (profiles/r9_scene_update.json, DESIGN.md "Scene updates"): rigid motions of
+// one instance by up to 50 % of the scene extent kept the refit within 0.5 % of the built cost on C3 and C5, while fresh builds
+// of the same moved scenes differed from each other by up to 4 %; a rebuild costs 1.4 ms (C3) / 91 ms (C5) of device time against
+// 7 ms for a C5 refit, and trace time follows the cost. 1.25 stays clear of build-to-build variation and rebuilds long before the
+// extra trace time of one frame exceeds the price of the rebuild.
+constexpr double REFIT_MAX_GROWTH = 1.25;
+RT_HD bool refit_needs_rebuild(double sah_refit, double sah_built, double max_growth = REFIT_MAX_GROWTH) {
+    return sah_refit > max_growth * sah_built;
 }
 
 }  // namespace rt

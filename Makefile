@@ -5,7 +5,8 @@ CSRC := $(PKG)/csrc
 NVCCFLAGS := -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -Xcompiler -fvisibility=hidden $(NVCCFLAGS_EXTRA)
 HDRS := $(wildcard $(CSRC)/*.h) $(CSRC)/kernels.cuh include/rtcuda.h
 
-all: $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so oracle_ref
+all: $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so \
+	tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so oracle_ref
 
 # the reference's own C++ device headers compiled for the host (checker of the oracle; no-op when /root/reference is absent)
 .PHONY: oracle_ref
@@ -42,5 +43,14 @@ tests/hostsim/libhostsim.so: tests/hostsim/hostsim.cpp $(HDRS)
 tests/hostsim/libhostsim_update.so: tests/hostsim/hostsim_update.cpp tests/hostsim/hostsim.cpp $(HDRS)
 	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
 
+# the ray queries on the CPU (includes hostsim.cpp)
+tests/hostsim/libhostsim_query.so: tests/hostsim/hostsim_query.cpp tests/hostsim/hostsim.cpp $(HDRS)
+	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
+
+# their reference: the oracle's traverse_bvh per caller-supplied ray (includes oracle/oracle.cpp, built with the oracle's flags)
+tests/hostsim/liboracle_query.so: tests/hostsim/oracle_query.cpp oracle/oracle.cpp include/rtcuda.h
+	g++ -O2 -std=c++17 -fPIC -ffp-contract=off -fno-fast-math -Wall -Wno-unused-function -pthread -shared -o $@ $<
+
 clean:
-	rm -rf build $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so
+	rm -rf build $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so \
+		tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so

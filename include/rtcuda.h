@@ -430,6 +430,35 @@ RTCUDA_API rtcuda_status rtcuda_render_pixel(rtcuda_scene* scene, const rtcuda_s
                                              uint32_t x, uint32_t y, uint32_t sample_lo, uint32_t sample_hi,
                                              rtcuda_pixel_output* out);
 
+/* Ray queries: caller-supplied rays against the uploaded scene's BVH (the analogue of Embree's rtcIntersect / rtcOccluded).
+ * `rays` is `count` x 8 floats per ray: origin.xyz, t_min, direction.xyz, t_max (32 bytes, the shape of the render's ray queue).
+ *   - Closest hit: the hit with the smallest t in [t_min, t_max]. Both bounds are inclusive, there is no back-face culling, and
+ *     equal-t ties go to the larger (geom_id, prim_id): the acceptance rule of the render's traversal. Triangles are tested with
+ *     the context's test (Moller-Trumbore, or Woop's watertight test under RTCUDA_BACKEND_WATERTIGHT). t is in units of the
+ *     direction's length (the direction is not normalised) and there is no implicit epsilon: a ray that starts on a surface
+ *     needs its own t_min offset.
+ *   - Outputs, each NULL to skip it (at least one must be given): t[i]; ids[2i] = instance index (geom_id), ids[2i+1] = primitive
+ *     index within the shape (prim_id; 0 for a sphere); barycentrics[2i], [2i+1] = (u, v), the weights of v1 and v2 (0 for a
+ *     sphere). The winning triangle is re-tested in object space like the first-hit AOVs, so t / u / v are the reference's
+ *     intersect_shape values to rounding.
+ *   - Miss: t = +INFINITY, both ids RTCUDA_NONE, barycentrics 0. A ray with t_min > t_max, a zero direction, a NaN bound or a
+ *     non-finite origin or direction component is a miss, not an error.
+ *   - Occlusion: occluded[i] = 1 when any primitive is hit in [t_min, t_max], else 0 (the any-hit walk of shadow rays).
+ *   - The plain variants take HOST arrays and block until the results are on the host; on a multi-device scene the rays are cut
+ *     into contiguous slices, one per GPU. The _device variants take DEVICE pointers on device_ids[0] (the context's GPU), rays
+ *     16-byte aligned, and block until the outputs are written. The library's stream does not wait for other streams: the caller
+ *     must have finished writing the rays (e.g. torch.cuda.synchronize()) before the call.
+ *   - count == 0 is RTCUDA_OK; count >= 2^32, NULL rays with count > 0, no output, or (device variants) a pointer that is not
+ *     device memory of that GPU are RTCUDA_ERR_INVALID_ARGUMENT, refused before any device work.
+ *   - Queries read the scene only: rtcuda_get_stats keeps reporting the last render, and nothing a render caches is touched.
+ * Results are the same bit for bit on one GPU, on several, and from host or device arrays. */
+RTCUDA_API rtcuda_status rtcuda_trace_rays(rtcuda_scene* scene, const float* rays, uint64_t count, float* t, uint32_t* ids,
+                                           float* barycentrics);
+RTCUDA_API rtcuda_status rtcuda_trace_rays_device(rtcuda_scene* scene, const float* rays, uint64_t count, float* t, uint32_t* ids,
+                                                  float* barycentrics);
+RTCUDA_API rtcuda_status rtcuda_occluded(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded);
+RTCUDA_API rtcuda_status rtcuda_occluded_device(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded);
+
 RTCUDA_API rtcuda_status rtcuda_get_stats(const rtcuda_scene* scene, rtcuda_stats* out);
 
 /* Message of the last failing call on this thread ("" if none). */

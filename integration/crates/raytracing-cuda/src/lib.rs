@@ -451,6 +451,43 @@ impl CudaScene {
     }
 }
 
+/// Closest hit of one query ray (`rtcuda_trace_rays`): `t` is +inf and both ids `RTCUDA_NONE` on a miss; `barycentrics` are
+/// the weights of the triangle's v1 and v2 (0 for spheres and misses).
+#[derive(Clone, Copy, Debug, PartialEq)]
+pub struct RayHit {
+    pub t: f32,
+    pub geom_id: u32,
+    pub prim_id: u32,
+    pub barycentrics: [f32; 2],
+}
+
+impl CudaScene {
+    /// Closest hit of every ray in [t_min, t_max] (`[origin.xyz, t_min, direction.xyz, t_max]`): both bounds inclusive, no
+    /// back-face culling, equal-t ties to the larger (geom_id, prim_id). The direction is not normalised (t is in its units).
+    pub fn trace_rays(&self, rays: &[[f32; 8]]) -> Vec<RayHit> {
+        let n = rays.len();
+        let mut t = vec![0.0f32; n];
+        let mut ids = vec![0u32; 2 * n];
+        let mut uv = vec![0.0f32; 2 * n];
+        // SAFETY: [f32; 8] is 8 packed floats; the outputs are sized for n rays; the call blocks until they are written
+        unsafe {
+            check(ffi::rtcuda_trace_rays(self.scene, rays.as_ptr() as *const f32, n as u64, t.as_mut_ptr(), ids.as_mut_ptr(), uv.as_mut_ptr()),
+                  "rtcuda_trace_rays");
+        }
+        (0..n).map(|i| RayHit { t: t[i], geom_id: ids[2 * i], prim_id: ids[2 * i + 1], barycentrics: [uv[2 * i], uv[2 * i + 1]] }).collect()
+    }
+
+    /// Whether anything is hit in [t_min, t_max] along each ray (`rtcuda_occluded`, the any-hit walk of shadow rays).
+    pub fn occluded(&self, rays: &[[f32; 8]]) -> Vec<bool> {
+        let mut occ = vec![0u8; rays.len()];
+        // SAFETY: as in trace_rays
+        unsafe {
+            check(ffi::rtcuda_occluded(self.scene, rays.as_ptr() as *const f32, rays.len() as u64, occ.as_mut_ptr()), "rtcuda_occluded");
+        }
+        occ.into_iter().map(|o| o != 0).collect()
+    }
+}
+
 impl Drop for CudaScene {
     fn drop(&mut self) {
         // SAFETY: handles created by rtcuda_init / rtcuda_scene_upload, released exactly once

@@ -6,7 +6,7 @@ from .renderer import AovFlags, RaytracerSettings, RenderOutput, Sampler, Single
 from .scene import (Camera, Light, Material, Mesh, Scene, SceneBuilder, Sphere, Texture, scene_from_gltf_file,
                     mesh_from_ply_bytes)
 from .pbrt import scene_from_pbrt_file, scene_from_pbrt_string, PbrtParseError
-from .backend import CudaBackendSettings, CudaRenderer, render, render_single_pixel
+from .backend import CudaBackendSettings, CudaRenderer, RayHits, make_rays, render, render_single_pixel
 from . import test_scenes
 from . import multi_gpu
 from . import exr
@@ -14,5 +14,5 @@ from . import imagecmp
 
 __all__ = ["AovFlags", "RaytracerSettings", "RenderOutput", "Sampler", "SinglePixelOutput", "Camera", "Light",
            "Material", "Mesh", "Scene", "SceneBuilder", "Sphere", "Texture", "scene_from_gltf_file", "scene_from_pbrt_file", "scene_from_pbrt_string", "PbrtParseError",
-           "mesh_from_ply_bytes", "CudaBackendSettings", "CudaRenderer", "render", "render_single_pixel",
+           "mesh_from_ply_bytes", "CudaBackendSettings", "CudaRenderer", "RayHits", "make_rays", "render", "render_single_pixel",
            "test_scenes"]

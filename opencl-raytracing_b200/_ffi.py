@@ -144,7 +144,8 @@ ABI_STRUCTS = [Camera, Shape, Instance, Light, Material, Texture, Image, SceneDe
 # every symbol include/rtcuda.h declares
 EXPORTED_SYMBOLS = ["rtcuda_init", "rtcuda_shutdown", "rtcuda_scene_upload", "rtcuda_scene_update", "rtcuda_scene_release", "rtcuda_release_cached_memory", "rtcuda_render",
                     "rtcuda_render_device", "rtcuda_render_samples_device", "rtcuda_render_samples_accumulate_device", "rtcuda_render_pixel", "rtcuda_get_stats", "rtcuda_last_error",
-                    "rtcuda_abi_version", "rtcuda_abi_struct_sizes", "rtcuda_host_alloc", "rtcuda_host_free"]
+                    "rtcuda_abi_version", "rtcuda_abi_struct_sizes", "rtcuda_host_alloc", "rtcuda_host_free", "rtcuda_trace_rays",
+                    "rtcuda_trace_rays_device", "rtcuda_occluded", "rtcuda_occluded_device"]
 
 _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG_DIR, "libraytracing_cuda.so")
@@ -194,6 +195,15 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.rtcuda_render_pixel.argtypes = [C.c_void_p, C.POINTER(Settings), C.c_uint32, C.c_uint32, C.c_uint32,
                                         C.c_uint32, C.POINTER(PixelOutput)]
     lib.rtcuda_render_pixel.restype = C.c_int
+    # ray queries: scene, rays (count x 8 floats), count, then the outputs (host or device addresses; None = skip)
+    lib.rtcuda_trace_rays.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.rtcuda_trace_rays.restype = C.c_int
+    lib.rtcuda_trace_rays_device.argtypes = lib.rtcuda_trace_rays.argtypes
+    lib.rtcuda_trace_rays_device.restype = C.c_int
+    lib.rtcuda_occluded.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]
+    lib.rtcuda_occluded.restype = C.c_int
+    lib.rtcuda_occluded_device.argtypes = lib.rtcuda_occluded.argtypes
+    lib.rtcuda_occluded_device.restype = C.c_int
     lib.rtcuda_get_stats.argtypes = [C.c_void_p, C.POINTER(Stats)]
     lib.rtcuda_get_stats.restype = C.c_int
     lib.rtcuda_last_error.argtypes = []

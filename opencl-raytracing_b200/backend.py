@@ -51,6 +51,45 @@ class CudaBackendSettings:
         return b
 
 
+def make_rays(origins, directions, t_min=0.0, t_max=np.inf) -> np.ndarray:
+    """Pack rays for CudaRenderer.trace / occluded: float32 [N, 8] rows of origin.xyz, t_min, direction.xyz, t_max. `origins` and
+    `directions` are [N, 3] (or one [3] row, broadcast); t_min / t_max are scalars or [N]. Directions are not normalised: hit
+    t is in units of the direction's length."""
+    o = np.asarray(origins, dtype=np.float32)
+    d = np.asarray(directions, dtype=np.float32)
+    if o.shape[-1:] != (3,) or d.shape[-1:] != (3,) or o.ndim > 2 or d.ndim > 2:
+        raise ValueError(f"origins and directions must be [N, 3] or [3], got {o.shape} and {d.shape}")
+    n = max(o.shape[0] if o.ndim == 2 else 1, d.shape[0] if d.ndim == 2 else 1)
+    rays = np.empty((n, 8), dtype=np.float32)
+    try:
+        rays[:, 0:3] = o
+        rays[:, 4:7] = d
+        rays[:, 3] = np.asarray(t_min, dtype=np.float32)
+        rays[:, 7] = np.asarray(t_max, dtype=np.float32)
+    except ValueError as e:
+        raise ValueError(f"ray fields do not broadcast to {n} rays: {e}") from None
+    return rays
+
+
+@dataclass
+class RayHits:
+    """Closest hits of CudaRenderer.trace, one row per ray: t (+inf on a miss), the instance index (geom_id) and the primitive
+    index within its shape (prim_id, 0 for a sphere) as uint32 (_ffi.NONE on a miss), and the barycentrics (u, v) = the
+    weights of the triangle's v1 and v2 (0 for spheres and misses)."""
+    t: np.ndarray              # float32 [N]
+    instance: np.ndarray       # uint32 [N]
+    primitive: np.ndarray      # uint32 [N]
+    barycentrics: np.ndarray   # float32 [N, 2]
+
+
+def _check_rays(rays) -> np.ndarray:
+    if not isinstance(rays, np.ndarray) or rays.dtype != np.float32 or rays.ndim != 2 or rays.shape[1] != 8:
+        raise ValueError("rays must be a float32 numpy array of shape [N, 8] (see make_rays)")
+    if not rays.flags.c_contiguous:
+        raise ValueError("rays must be C-contiguous")
+    return rays
+
+
 def warn_nonfinite(beauty: np.ndarray, log=None) -> int:
     """The tail of raytracing_cpu::render (lib.rs:813-854): every channel of the beauty plane is classified, the first 10
     NaN / infinite ones are reported in raster order, then the total. The count comes from the device (k_finalize); this
@@ -165,6 +204,39 @@ class CudaRenderer:
         _ffi.check(self.lib, self.lib.rtcuda_render_pixel(self._scene, C.byref(s), x, y, sample_lo, sample_hi, buf),
                    "rtcuda_render_pixel")
         return [SinglePixelOutput(b.sample_index, bool(b.hit), tuple(b.uv), tuple(b.normal), tuple(b.radiance)) for b in buf[:n]]
+
+    def trace(self, rays: np.ndarray) -> RayHits:
+        """Closest hit of every ray of `rays` (float32 [N, 8], make_rays) in [t_min, t_max], both inclusive, no back-face
+        culling; equal-t ties go to the larger (instance, primitive). Host arrays; blocks until the results are here. Queries
+        leave the render state and stats() alone."""
+        rays = _check_rays(rays)
+        n = rays.shape[0]
+        t = np.empty(n, np.float32)
+        ids = np.empty((n, 2), np.uint32)
+        uv = np.empty((n, 2), np.float32)
+        _ffi.check(self.lib, self.lib.rtcuda_trace_rays(self._scene, rays.ctypes.data, n, t.ctypes.data, ids.ctypes.data, uv.ctypes.data),
+                   "rtcuda_trace_rays")
+        return RayHits(t, ids[:, 0].copy(), ids[:, 1].copy(), uv)
+
+    def occluded(self, rays: np.ndarray) -> np.ndarray:
+        """bool [N]: whether anything is hit in [t_min, t_max] (the any-hit walk of shadow rays)."""
+        rays = _check_rays(rays)
+        occ = np.empty(rays.shape[0], np.uint8)
+        _ffi.check(self.lib, self.lib.rtcuda_occluded(self._scene, rays.ctypes.data, rays.shape[0], occ.ctypes.data), "rtcuda_occluded")
+        return occ.view(np.bool_)
+
+    def trace_device(self, rays_ptr: int, count: int, t_ptr: Optional[int] = None, ids_ptr: Optional[int] = None,
+                     barycentrics_ptr: Optional[int] = None) -> None:
+        """trace() on DEVICE arrays of the context's first GPU (e.g. torch tensors' data_ptr()): rays count x 8 float32, 16-byte
+        aligned; t count float32, ids count x 2 uint32 (int32 tensors work), barycentrics count x 2 float32; None skips an output.
+        The library's stream does not wait for the caller's: finish writing the rays first (torch.cuda.synchronize()). Blocks
+        until the outputs are written."""
+        _ffi.check(self.lib, self.lib.rtcuda_trace_rays_device(self._scene, rays_ptr, count, t_ptr, ids_ptr, barycentrics_ptr),
+                   "rtcuda_trace_rays_device")
+
+    def occluded_device(self, rays_ptr: int, count: int, occluded_ptr: int) -> None:
+        """occluded() on DEVICE arrays (see trace_device): one uint8 per ray, 1 = occluded."""
+        _ffi.check(self.lib, self.lib.rtcuda_occluded_device(self._scene, rays_ptr, count, occluded_ptr), "rtcuda_occluded_device")
 
     def stats(self) -> dict:
         st = _ffi.Stats()

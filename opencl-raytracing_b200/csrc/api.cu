@@ -1553,6 +1553,99 @@ void render_pixel(rtcuda_scene* s, const rtcuda_settings* settings, uint32_t x, 
     CK(cudaStreamSynchronize(st));
 }
 
+// ---------------------------------------------------------------------------------------------------
+// ray queries (rtcuda_trace_rays / rtcuda_occluded): caller-supplied rays against the scene's BVH
+// ---------------------------------------------------------------------------------------------------
+// A query reads the scene and nothing else: no stats, no frame graph, no pixel lists, no path-state arena. Its scratch comes from
+// the stream-ordered pool, sized for one chunk of rays.
+constexpr uint64_t QUERY_CHUNK = 1ull << 24;   // rays per launch: 512 MB of rays and 256 MB of scratch hits
+
+// Query outputs as the C ABI takes them (occluded set: an occlusion query; otherwise a closest-hit query)
+struct QueryPtrs {
+    const float* rays;
+    float* t;
+    uint32_t* ids;
+    float* uv;
+    uint8_t* occluded;
+};
+
+// Checks that need no device: done first, so that a refused query does no device work
+void validate_query(const rtcuda_scene* s, const QueryPtrs& q, uint64_t count) {
+    REQUIRE(count < (1ull << 32), "ray count must be below 2^32");
+    REQUIRE(q.rays || count == 0, "rays is NULL");
+    REQUIRE(q.t || q.ids || q.uv || q.occluded, "every output is NULL");
+    REQUIRE(s, "scene is NULL");
+}
+
+// Pointers of the device variants must be device (or managed) memory of the GPU the scene's first context runs on
+void require_device_pointer(const void* p, int device, const char* what) {
+    if (!p) return;
+    cudaPointerAttributes a{};
+    const cudaError_t e = cudaPointerGetAttributes(&a, p);
+    if (e != cudaSuccess) cudaGetLastError();
+    REQUIRE(e == cudaSuccess && (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == device,
+            std::string(what) + " is not device memory of device " + std::to_string(device));
+}
+
+// Kernels of one chunk: rays and outputs are device pointers already offset to the chunk
+void query_chunk(rtcuda_scene* s, const float4* rays, uint32_t n, const QueryPtrs& out, float4* hits, uint32_t* counter, LaunchCounter& lc) {
+    cudaStream_t st = s->ctx->stream;
+    CK(cudaMemsetAsync(counter, 0, sizeof(uint32_t), st));
+    if (out.occluded) {
+        launch_occluded(st, s->sc, rays, n, out.occluded, counter, lc);
+        return;
+    }
+    launch_trace(st, s->sc, rays, n, hits, counter, lc);
+    launch_trace_finish(st, s->sc, rays, hits, n, QueryOut{out.t, out.ids, out.uv}, lc);
+}
+
+// Device arrays on this scene's GPU; blocks until the outputs are written
+void query_device(rtcuda_scene* s, const QueryPtrs& q, uint64_t count) {
+    LaunchCounter lc;   // (not the scene's: the stats keep describing the last render)
+    DevBuf<uint32_t> counter;
+    DevBuf<float4> hits;
+    counter.alloc(1);
+    if (!q.occluded) hits.alloc(std::min(count, QUERY_CHUNK));
+    for (uint64_t b = 0; b < count; b += QUERY_CHUNK) {
+        const uint32_t n = (uint32_t)std::min(QUERY_CHUNK, count - b);
+        const QueryPtrs o{nullptr, q.t ? q.t + b : nullptr, q.ids ? q.ids + 2 * b : nullptr, q.uv ? q.uv + 2 * b : nullptr,
+                          q.occluded ? q.occluded + b : nullptr};
+        query_chunk(s, (const float4*)q.rays + 2 * b, n, o, hits.p, counter.p, lc);
+    }
+    CK(cudaStreamSynchronize(s->ctx->stream));
+}
+
+// Host arrays: per chunk, rays in, kernels, requested outputs out (cudaMemcpyAsync on the scene's stream); blocks until the
+// results are on the host
+void query_host(rtcuda_scene* s, const QueryPtrs& q, uint64_t count) {
+    cudaStream_t st = s->ctx->stream;
+    LaunchCounter lc;
+    const uint64_t cap = std::min(count, QUERY_CHUNK);
+    DevBuf<uint32_t> counter;
+    DevBuf<float4> rays, hits;
+    DevBuf<float> t, uv;
+    DevBuf<uint32_t> ids;
+    DevBuf<uint8_t> occ;
+    counter.alloc(1);
+    rays.alloc(2 * cap);
+    if (q.occluded) occ.alloc(cap);
+    else hits.alloc(cap);
+    if (q.t) t.alloc(cap);
+    if (q.ids) ids.alloc(2 * cap);
+    if (q.uv) uv.alloc(2 * cap);
+    const QueryPtrs dev{nullptr, q.t ? t.p : nullptr, q.ids ? ids.p : nullptr, q.uv ? uv.p : nullptr, q.occluded ? occ.p : nullptr};
+    for (uint64_t b = 0; b < count; b += QUERY_CHUNK) {
+        const uint32_t n = (uint32_t)std::min(QUERY_CHUNK, count - b);
+        CK(cudaMemcpyAsync(rays.p, q.rays + 8 * b, (size_t)n * 32, cudaMemcpyHostToDevice, st));
+        query_chunk(s, rays.p, n, dev, hits.p, counter.p, lc);
+        if (q.t) CK(cudaMemcpyAsync(q.t + b, t.p, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+        if (q.ids) CK(cudaMemcpyAsync(q.ids + 2 * b, ids.p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+        if (q.uv) CK(cudaMemcpyAsync(q.uv + 2 * b, uv.p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+        if (q.occluded) CK(cudaMemcpyAsync(q.occluded + b, occ.p, (size_t)n, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
+}
+
 
 // ---------------------------------------------------------------------------------------------------
 // scene update: camera, instance transforms and lights of an uploaded scene, in place
@@ -1992,6 +2085,21 @@ void multi_render_device(rtcuda_scene* parent, const rtcuda_settings* settings, 
     CK(cudaStreamSynchronize(st0));
 }
 
+// Host-array queries on a multi-device scene: contiguous slices of the rays, one per GPU, each on its own host thread. Every ray is
+// traced on a replica of the same tree, so the results are those of one GPU.
+void multi_query_host(rtcuda_scene* parent, const QueryPtrs& q, uint64_t count) {
+    const size_t n = parent->subs.size();
+    const uint64_t per = (count + n - 1) / n;
+    for_each_device(n, [&](size_t r) {
+        const uint64_t lo = std::min<uint64_t>(count, per * r), hi = std::min<uint64_t>(count, lo + per);
+        if (hi == lo) return;
+        enter(parent->subs[r]);
+        const QueryPtrs slice{q.rays + 8 * lo, q.t ? q.t + lo : nullptr, q.ids ? q.ids + 2 * lo : nullptr, q.uv ? q.uv + 2 * lo : nullptr,
+                              q.occluded ? q.occluded + lo : nullptr};
+        query_host(parent->subs[r], slice, hi - lo);
+    });
+}
+
 // rtcuda_get_stats of a multi-device scene: ray / fetch / launch counters summed over the GPUs, times = the slowest GPU
 rtcuda_stats multi_stats(const rtcuda_scene* parent) {
     rtcuda_stats t{};
@@ -2264,6 +2372,41 @@ RTCUDA_API rtcuda_status rtcuda_render_pixel(rtcuda_scene* scene, const rtcuda_s
         tls_stream = one->ctx->stream;
         render_pixel(one, settings, x, y, sample_lo, sample_hi, out);
     });
+}
+
+namespace {
+rtcuda_status query(rtcuda_scene* scene, const QueryPtrs& q, uint64_t count, bool device_arrays) {
+    return guarded([&] {
+        validate_query(scene, q, count);
+        if (count == 0) return;
+        if (!device_arrays && !scene->subs.empty()) { multi_query_host(scene, q, count); return; }
+        rtcuda_scene* one = scene->subs.empty() ? scene : scene->subs[0];   // device arrays live on device_ids[0]
+        CK(cudaSetDevice(one->ctx->device));
+        tls_stream = one->ctx->stream;
+        if (!device_arrays) { query_host(one, q, count); return; }
+        REQUIRE(((uintptr_t)q.rays & 15u) == 0, "rays must be 16-byte aligned");
+        require_device_pointer(q.rays, one->ctx->device, "rays");
+        require_device_pointer(q.t, one->ctx->device, "t");
+        require_device_pointer(q.ids, one->ctx->device, "ids");
+        require_device_pointer(q.uv, one->ctx->device, "barycentrics");
+        require_device_pointer(q.occluded, one->ctx->device, "occluded");
+        query_device(one, q, count);
+    });
+}
+}  // namespace
+
+RTCUDA_API rtcuda_status rtcuda_trace_rays(rtcuda_scene* scene, const float* rays, uint64_t count, float* t, uint32_t* ids, float* barycentrics) {
+    return query(scene, QueryPtrs{rays, t, ids, barycentrics, nullptr}, count, false);
+}
+RTCUDA_API rtcuda_status rtcuda_trace_rays_device(rtcuda_scene* scene, const float* rays, uint64_t count, float* t, uint32_t* ids,
+                                                  float* barycentrics) {
+    return query(scene, QueryPtrs{rays, t, ids, barycentrics, nullptr}, count, true);
+}
+RTCUDA_API rtcuda_status rtcuda_occluded(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded) {
+    return query(scene, QueryPtrs{rays, nullptr, nullptr, nullptr, occluded}, count, false);
+}
+RTCUDA_API rtcuda_status rtcuda_occluded_device(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded) {
+    return query(scene, QueryPtrs{rays, nullptr, nullptr, nullptr, occluded}, count, true);
 }
 
 RTCUDA_API rtcuda_status rtcuda_get_stats(const rtcuda_scene* scene, rtcuda_stats* out) {

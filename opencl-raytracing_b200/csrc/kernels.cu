@@ -337,6 +337,58 @@ __global__ void __launch_bounds__(BLOCK, SHADOW_BLOCKS) k_shadow(const __grid_co
     }
 }
 
+// Ray queries (rtcuda_trace_rays / rtcuda_occluded): caller-supplied rays (rt_query.h), closest hit or any hit, with the
+// refill / phase-vote loop of k_extend and k_shadow. The loop is duplicated here on purpose: folding the three kernels onto one
+// loop would make the renderer's hottest kernels branch on their caller and change their SASS. Launch bounds follow the
+// kernel each variant mirrors. Closest hit writes the traversal's Hit per ray (k_trace_finish turns it into ids and the
+// object-space t / u / v); any hit writes the occlusion byte.
+template <bool ANY_HIT>
+__global__ void __launch_bounds__(BLOCK, ANY_HIT ? SHADOW_BLOCKS : 4) k_trace(const __grid_constant__ SceneD sc, const float4* __restrict__ rays,
+                                                                            uint32_t n, float4* hits, uint8_t* occluded, uint32_t* fetch_counter) {
+    const unsigned FULL = 0xffffffffu;
+    const unsigned lane = threadIdx.x & 31u, lt = (1u << lane) - 1u;
+    uint2 stack_mem[TRAVERSE_STACK];
+    Traversal<ANY_HIT, false> tr;
+    tr.stack = stack_mem;
+    uint32_t have = 0u, exhausted = n == 0 ? 1u : 0u;
+    uint32_t q = 0;
+    for (;;) {
+        const unsigned need = __ballot_sync(FULL, !have);
+        if (need == FULL && exhausted) break;
+        if (!exhausted && __popc(need) >= REFILL_MIN) {
+            const int cnt = __popc(need), leader = __ffs(need) - 1;
+            uint32_t base = 0;
+            if ((int)lane == leader) base = atomicAdd(fetch_counter, (uint32_t)cnt);
+            base = __shfl_sync(FULL, base, leader);
+            if (!have) {
+                const uint32_t mine = base + (uint32_t)__popc(need & lt);
+#if RT_REFILL_PREFETCH
+                {
+                    const uint32_t ahead = mine + (uint32_t)RT_REFILL_PREFETCH * gridDim.x * BLOCK;
+                    if (ahead < n) prefetch_l2(rays + 2 * (size_t)ahead);   // both halves of a ray share a 32-byte sector
+                }
+#endif
+                if (mine < n) {
+                    q = mine;
+                    const float4 o4 = ld_stream(&rays[2 * (size_t)q]), d4 = ld_stream(&rays[2 * (size_t)q + 1]);
+                    have = query_ray_valid(o4, d4) && tr.init(sc, xyz(o4), xyz(d4), o4.w, d4.w) ? 1u : 0u;
+                    if (!have) {
+                        if (ANY_HIT) occluded[q] = 0u;
+                        else st_stream(&hits[q], query_miss_entry());
+                    }
+                }
+            }
+            if (base + (uint32_t)cnt >= n) exhausted = 1u;
+        }
+        warp_phase(tr, have, sc, (TraverseStats*)nullptr);
+        if (have && !tr.next()) {
+            if (ANY_HIT) occluded[q] = tr.found ? 1u : 0u;
+            else st_stream(&hits[q], tr.found ? query_hit_entry(tr.hit) : query_miss_entry());
+            have = 0u;
+        }
+    }
+}
+
 __global__ void __launch_bounds__(BLOCK) k_shadow_gather(const __grid_constant__ Wave w) {
     const uint32_t n = (uint32_t)(*w.n_shadow & 0xffffffffull);
     for (uint32_t v = blockIdx.x * BLOCK + threadIdx.x; v < n; v += gridDim.x * BLOCK) shadow_gather_body(v, w);
@@ -406,6 +458,15 @@ void launch_shade(cudaStream_t st, const SceneD& sc, const RenderParams& rp, con
 void launch_shadow(cudaStream_t st, const SceneD& sc, const Wave& w, uint32_t n_max, uint32_t* fetch_counter, bool stats, LaunchCounter& lc) {
     if (stats) k_shadow<true><<<persistent_grid((const void*)k_shadow<true>, n_max), BLOCK, 0, st>>>(sc, w, fetch_counter);
     else k_shadow<false><<<persistent_grid((const void*)k_shadow<false>, n_max), BLOCK, 0, st>>>(sc, w, fetch_counter);
+    lc.launches++;
+}
+void launch_trace(cudaStream_t st, const SceneD& sc, const float4* rays, uint32_t n, float4* hits, uint32_t* fetch_counter, LaunchCounter& lc) {
+    k_trace<false><<<persistent_grid((const void*)k_trace<false>, n), BLOCK, 0, st>>>(sc, rays, n, hits, nullptr, fetch_counter);
+    lc.launches++;
+}
+void launch_occluded(cudaStream_t st, const SceneD& sc, const float4* rays, uint32_t n, uint8_t* occluded, uint32_t* fetch_counter,
+                     LaunchCounter& lc) {
+    k_trace<true><<<persistent_grid((const void*)k_trace<true>, n), BLOCK, 0, st>>>(sc, rays, n, nullptr, occluded, fetch_counter);
     lc.launches++;
 }
 void launch_shadow_gather(cudaStream_t st, const Wave& w, uint32_t n_max, LaunchCounter& lc) {

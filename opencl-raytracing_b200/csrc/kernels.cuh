@@ -2,6 +2,7 @@
 #pragma once
 #include "rt_build.h"
 #include "rt_integrator.h"
+#include "rt_query.h"
 
 namespace rt {
 
@@ -33,6 +34,14 @@ struct PixelOut { uint32_t sample_index, hit; float uv[2]; float normal[3]; floa
 void launch_pixel_aov(cudaStream_t st, const SceneD& sc, const RenderParams& rp, uint32_t x, uint32_t y, uint32_t sample_lo,
                       uint32_t n, PixelOut* out, LaunchCounter& lc);
 void launch_pixel_radiance(cudaStream_t st, const float4* radiance, uint32_t n, PixelOut* out, LaunchCounter& lc);
+
+// ray queries (rtcuda_trace_rays / rtcuda_occluded): persistent traversal of n packed rays (rt_query.h), then, for closest hits,
+// one thread per ray for the ids and the object-space re-test. `fetch_counter` must be zero.
+void launch_trace(cudaStream_t st, const SceneD& sc, const float4* rays, uint32_t n, float4* hits, uint32_t* fetch_counter, LaunchCounter& lc);
+void launch_occluded(cudaStream_t st, const SceneD& sc, const float4* rays, uint32_t n, uint8_t* occluded, uint32_t* fetch_counter,
+                     LaunchCounter& lc);
+void launch_trace_finish(cudaStream_t st, const SceneD& sc, const float4* rays, const float4* hits, uint32_t n, const QueryOut& out,
+                         LaunchCounter& lc);
 
 // BVH build
 void launch_prim_setup(cudaStream_t st, const BuildCtx& b, LaunchCounter& lc);

@@ -46,6 +46,20 @@ __global__ void k_pixel_radiance(const float4* radiance, uint32_t n, PixelOut* o
     out[i].radiance[0] = radiance[i].x; out[i].radiance[1] = radiance[i].y; out[i].radiance[2] = radiance[i].z;
 }
 
+// Ray queries, after k_trace (kernels.cu): here, in the IEEE translation unit, so that the re-test of the winning triangle reports
+// the reference's object-space t / u / v to rounding like the first-hit AOVs
+__global__ void __launch_bounds__(BLOCK) k_trace_finish(const __grid_constant__ SceneD sc, const float4* rays, const float4* hits, uint32_t n,
+                                                         const QueryOut out) {
+    const uint32_t i = blockIdx.x * BLOCK + threadIdx.x;
+    if (i < n) trace_finish_body(i, sc, rays, hits, out);
+}
+
+void launch_trace_finish(cudaStream_t st, const SceneD& sc, const float4* rays, const float4* hits, uint32_t n, const QueryOut& out,
+                         LaunchCounter& lc) {
+    k_trace_finish<<<grid_for(n), BLOCK, 0, st>>>(sc, rays, hits, n, out);
+    lc.launches++;
+}
+
 void launch_aov(cudaStream_t st, const SceneD& sc, const RenderParams& rp, const uint32_t* pixel_list, uint32_t n_pixels,
                 const AovPlanes& planes, unsigned long long* stats, bool collect, LaunchCounter& lc) {
     if (collect) k_aov<true><<<grid_for(n_pixels), BLOCK, 0, st>>>(sc, rp, pixel_list, n_pixels, planes, stats);

@@ -652,7 +652,8 @@ struct FirstHit { bool hit; V2 uv; V3 normal, albedo; bool has_mip; float mip; u
 // seen from 4 m resolves its hit point to ~1e-6, i.e. ~2e-4 of its edge) — visible in the uv AOV of meshes without uvs, where
 // uv IS the barycentrics. The first-hit AOV pass (one ray per pixel) therefore repeats the test of the WINNING triangle the
 // reference's way and reports those (t, u, v): same operations in the same order, un-fused in this translation unit.
-RT_HD void refine_triangle_hit_in_object_space(const SceneD& sc, const Ray& ray, Hit& h) {
+// [t_min, t_max] is the range the ray was traced over (the camera clip for first hits, the caller's range for ray queries).
+RT_HD void refine_triangle_hit_in_object_space(const SceneD& sc, const Ray& ray, float t_min, float t_max, Hit& h) {
     const Prim* pr = sc.prims + h.prim;
     if (f2u(ldg(&pr->c).w) != 0u) return;   // spheres are intersected in object space already
     const uint32_t geom = f2u(ldg(&pr->a).w), prim_id = f2u(ldg(&pr->b).w);
@@ -662,8 +663,8 @@ RT_HD void refine_triangle_hit_in_object_space(const SceneD& sc, const Ray& ray,
              p2 = load3(sc.vertices, inst.vertex_offset + ldg(t3 + 2));
     const V3 oo = apply_point(inst.w2o, ray.o), od = apply_vector(inst.w2o, ray.d);
     float t, u, v;
-    const bool ok = sc.watertight ? triangle_watertight(p0, p1, p2, oo, od, sc.camera.near_clip, sc.camera.far_clip, t, u, v)
-                                  : triangle_t(p0, p1, p2, oo, od, sc.camera.near_clip, sc.camera.far_clip, t, u, v);
+    const bool ok = sc.watertight ? triangle_watertight(p0, p1, p2, oo, od, t_min, t_max, t, u, v)
+                                  : triangle_t(p0, p1, p2, oo, od, t_min, t_max, t, u, v);
     if (ok) { h.t = t; h.u = u; h.v = v; }
 }
 
@@ -680,7 +681,7 @@ RT_HD FirstHit first_hit(const SceneD& sc, const RenderParams& rp, uint32_t px, 
     r.geom = NONE; r.prim = NONE; r.t = 0.0f;
     Hit h;
     if (!traverse<false, STATS>(sc, ray.o, ray.d, sc.camera.near_clip, sc.camera.far_clip, h, stats)) return r;
-    refine_triangle_hit_in_object_space(sc, ray, h);
+    refine_triangle_hit_in_object_space(sc, ray, sc.camera.near_clip, sc.camera.far_clip, h);
     HitInfo hit;
     reconstruct_hit(sc, ray.o, ray.d, h, true, hit);
     MatCtx mc = matctx_from_differentials(hit, ray, rd);

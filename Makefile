@@ -6,7 +6,8 @@ NVCCFLAGS := -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -X
 HDRS := $(wildcard $(CSRC)/*.h) $(CSRC)/kernels.cuh include/rtcuda.h
 
 all: $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so \
-	tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so oracle_ref
+	tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so tests/hostsim/libhostsim_radiance.so tests/hostsim/liboracle_radiance.so \
+	oracle_ref
 
 # the reference's own C++ device headers compiled for the host (checker of the oracle; no-op when /root/reference is absent)
 .PHONY: oracle_ref
@@ -51,6 +52,14 @@ tests/hostsim/libhostsim_query.so: tests/hostsim/hostsim_query.cpp tests/hostsim
 tests/hostsim/liboracle_query.so: tests/hostsim/oracle_query.cpp oracle/oracle.cpp include/rtcuda.h
 	g++ -O2 -std=c++17 -fPIC -ffp-contract=off -fno-fast-math -Wall -Wno-unused-function -pthread -shared -o $@ $<
 
+# radiance along caller-supplied rays on the CPU (includes hostsim.cpp)
+tests/hostsim/libhostsim_radiance.so: tests/hostsim/hostsim_radiance.cpp tests/hostsim/hostsim.cpp $(HDRS)
+	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
+
+# its reference: the oracle's ray_radiance per caller-supplied ray (includes oracle/oracle.cpp, built with the oracle's flags)
+tests/hostsim/liboracle_radiance.so: tests/hostsim/oracle_radiance.cpp oracle/oracle.cpp include/rtcuda.h
+	g++ -O2 -std=c++17 -fPIC -ffp-contract=off -fno-fast-math -Wall -Wno-unused-function -pthread -shared -o $@ $<
+
 clean:
 	rm -rf build $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so \
-		tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so
+		tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so tests/hostsim/libhostsim_radiance.so tests/hostsim/liboracle_radiance.so

@@ -459,6 +459,35 @@ RTCUDA_API rtcuda_status rtcuda_trace_rays_device(rtcuda_scene* scene, const flo
 RTCUDA_API rtcuda_status rtcuda_occluded(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded);
 RTCUDA_API rtcuda_status rtcuda_occluded_device(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded);
 
+/* Radiance along caller-supplied rays: the path tracer's estimate of the radiance arriving at each ray's origin from its direction
+ * (light probes, lightmap texels, cameras the scene format lacks, reference radiance along chosen rays).
+ *   - `rays` is `count` x 8 floats per ray, packed like the ray queries: origin.xyz, t_min, direction.xyz, t_max. The direction need
+ *     not have unit length: each ray is first normalised as len = sqrtf((dx*dx + dy*dy) + dz*dz), d' = d / len (one IEEE division
+ *     per component), t_min' = t_min * len, t_max' = t_max * len, and its first segment is traced over [t_min', t_max'].
+ *   - radiance[3i .. 3i+2] = the mean over samples [0, settings->samples_per_pixel) of the radiance the integrator carries back
+ *     along ray i: the renderer's path (emission, next-event estimation, every BSDF, textures, environment light), summed in
+ *     sample order and multiplied by 1 / spp like a pixel. A valid ray that hits nothing returns the environment radiance (0
+ *     without an environment light). An invalid ray (the ray-query rule: non-finite origin or direction, zero direction, NaN
+ *     bound, t_min > t_max; also a direction whose squared length is outside the float range) returns exactly 0 and is not traced.
+ *   - Settings used: max_ray_depth, accumulate_bounces, light_sample_count, samples_per_pixel, the seed and the sampler fields.
+ *     `outputs` is ignored, and antialias_primary_rays is treated as 0 (a caller's ray has no differentials).
+ *   - Sampler streams: sample s of ray i draws from the stream of the renderer's pixel (k & 0xffff, k >> 16) at sample s, with
+ *     k = stream_base + i; no camera numbers are drawn. So key k shares its numbers with that pixel at the same seed (callers who
+ *     combine both should use different seeds), and a ray's result depends only on the ray, its key, the settings and the scene:
+ *     not on chunking, batch sizes, GPU count or host vs device arrays. Slicing a ray set over calls with stream_base = the
+ *     slice's offset gives the bits of one call.
+ *   - rtcuda_radiance takes HOST arrays and blocks until the radiance is on the host; on a multi-device scene the rays are cut
+ *     into contiguous slices, one per GPU, each keeping its keys. rtcuda_radiance_device takes DEVICE pointers on device_ids[0],
+ *     rays 16-byte aligned, and blocks until the radiance is written; the caller must have finished writing the rays.
+ *   - count == 0 is RTCUDA_OK. count >= 2^32, stream_base + count > 2^32, NULL rays with count > 0, NULL radiance, NULL settings,
+ *     samples_per_pixel == 0, strata < 1 with the stratified sampler, or (device variant) a pointer that is not device memory of
+ *     that GPU are RTCUDA_ERR_INVALID_ARGUMENT, refused before any device work.
+ *   - rtcuda_get_stats keeps reporting the last render. The call may reuse (and grow) the scene's path-state memory. */
+RTCUDA_API rtcuda_status rtcuda_radiance(rtcuda_scene* scene, const rtcuda_settings* settings, const float* rays, uint64_t count,
+                                         uint32_t stream_base, float* radiance);
+RTCUDA_API rtcuda_status rtcuda_radiance_device(rtcuda_scene* scene, const rtcuda_settings* settings, const float* rays, uint64_t count,
+                                                uint32_t stream_base, float* radiance);
+
 RTCUDA_API rtcuda_status rtcuda_get_stats(const rtcuda_scene* scene, rtcuda_stats* out);
 
 /* Message of the last failing call on this thread ("" if none). */

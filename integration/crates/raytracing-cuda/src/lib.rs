@@ -486,6 +486,20 @@ impl CudaScene {
         }
         occ.into_iter().map(|o| o != 0).collect()
     }
+
+    /// The path tracer's mean radiance along every ray (`rtcuda_radiance`) over `settings.samples_per_pixel` samples. Directions
+    /// need not be unit length (the library normalises them and scales [t_min, t_max]); misses return the environment radiance
+    /// or 0, invalid rays 0. Sample s of ray i uses the sampler stream of pixel (k & 0xffff, k >> 16), k = stream_base + i.
+    pub fn radiance(&self, rays: &[[f32; 8]], settings: &RaytracerSettings, stream_base: u32) -> Vec<[f32; 3]> {
+        let mut out = vec![[0.0f32; 3]; rays.len()];
+        // SAFETY: [f32; 8] / [f32; 3] are packed floats; the output is sized for every ray; the call blocks until it is written
+        unsafe {
+            check(ffi::rtcuda_radiance(self.scene, &settings_to_c(settings), rays.as_ptr() as *const f32, rays.len() as u64, stream_base,
+                                       out.as_mut_ptr() as *mut f32),
+                  "rtcuda_radiance");
+        }
+        out
+    }
 }
 
 impl Drop for CudaScene {

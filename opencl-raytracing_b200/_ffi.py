@@ -145,7 +145,7 @@ ABI_STRUCTS = [Camera, Shape, Instance, Light, Material, Texture, Image, SceneDe
 EXPORTED_SYMBOLS = ["rtcuda_init", "rtcuda_shutdown", "rtcuda_scene_upload", "rtcuda_scene_update", "rtcuda_scene_release", "rtcuda_release_cached_memory", "rtcuda_render",
                     "rtcuda_render_device", "rtcuda_render_samples_device", "rtcuda_render_samples_accumulate_device", "rtcuda_render_pixel", "rtcuda_get_stats", "rtcuda_last_error",
                     "rtcuda_abi_version", "rtcuda_abi_struct_sizes", "rtcuda_host_alloc", "rtcuda_host_free", "rtcuda_trace_rays",
-                    "rtcuda_trace_rays_device", "rtcuda_occluded", "rtcuda_occluded_device"]
+                    "rtcuda_trace_rays_device", "rtcuda_occluded", "rtcuda_occluded_device", "rtcuda_radiance", "rtcuda_radiance_device"]
 
 _PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG_DIR, "libraytracing_cuda.so")
@@ -204,6 +204,11 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.rtcuda_occluded.restype = C.c_int
     lib.rtcuda_occluded_device.argtypes = lib.rtcuda_occluded.argtypes
     lib.rtcuda_occluded_device.restype = C.c_int
+    # radiance along rays: scene, settings, rays (count x 8 floats), count, stream_base, radiance (count x 3 floats)
+    lib.rtcuda_radiance.argtypes = [C.c_void_p, C.POINTER(Settings), C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p]
+    lib.rtcuda_radiance.restype = C.c_int
+    lib.rtcuda_radiance_device.argtypes = lib.rtcuda_radiance.argtypes
+    lib.rtcuda_radiance_device.restype = C.c_int
     lib.rtcuda_get_stats.argtypes = [C.c_void_p, C.POINTER(Stats)]
     lib.rtcuda_get_stats.restype = C.c_int
     lib.rtcuda_last_error.argtypes = []

@@ -238,6 +238,27 @@ class CudaRenderer:
         """occluded() on DEVICE arrays (see trace_device): one uint8 per ray, 1 = occluded."""
         _ffi.check(self.lib, self.lib.rtcuda_occluded_device(self._scene, rays_ptr, count, occluded_ptr), "rtcuda_occluded_device")
 
+    def radiance(self, rays: np.ndarray, settings: RaytracerSettings, stream_base: int = 0) -> np.ndarray:
+        """float32 [N, 3]: the path tracer's mean radiance along every ray of `rays` (float32 [N, 8], make_rays) over
+        settings.samples_per_pixel samples (rtcuda_radiance). Directions need not be unit length: each ray is normalised and
+        its range scaled by the direction's length. Misses return the environment radiance (or 0); invalid rays return 0.
+        Sample s of ray i uses the sampler stream of pixel (k & 0xffff, k >> 16), k = stream_base + i, so slicing a ray set
+        over calls with stream_base = the slice's offset reproduces one call bit for bit. Host arrays; blocks. stats() keeps
+        describing the last render."""
+        rays = _check_rays(rays)
+        out = np.empty((rays.shape[0], 3), np.float32)
+        s = settings.to_c()
+        _ffi.check(self.lib, self.lib.rtcuda_radiance(self._scene, C.byref(s), rays.ctypes.data, rays.shape[0], stream_base, out.ctypes.data),
+                   "rtcuda_radiance")
+        return out
+
+    def radiance_device(self, rays_ptr: int, count: int, settings: RaytracerSettings, radiance_ptr: int, stream_base: int = 0) -> None:
+        """radiance() on DEVICE arrays of the context's first GPU (e.g. torch tensors' data_ptr()): rays count x 8 float32, 16-byte
+        aligned; radiance count x 3 float32. Finish writing the rays first (torch.cuda.synchronize()). Blocks until written."""
+        s = settings.to_c()
+        _ffi.check(self.lib, self.lib.rtcuda_radiance_device(self._scene, C.byref(s), rays_ptr, count, stream_base, radiance_ptr),
+                   "rtcuda_radiance_device")
+
     def stats(self) -> dict:
         st = _ffi.Stats()
         _ffi.check(self.lib, self.lib.rtcuda_get_stats(self._scene, C.byref(st)), "rtcuda_get_stats")

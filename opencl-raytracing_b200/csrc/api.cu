@@ -1165,11 +1165,12 @@ size_t arena_bytes(size_t cap, uint32_t shadow_k, uint32_t max_depth) {
     return cap * (16 + 16 * 7 + 16 + 4) + cap * k * 48 + n_counters * 4 + ((size_t)max_depth + 3) * 8 + 16 * 256;
 }
 
-// Allocate the wavefront state for `capacity` path slots.
-void ensure_wave(rtcuda_scene* s, uint32_t capacity, uint32_t shadow_k, uint32_t max_depth) {
+// Allocate the wavefront state for `capacity` path slots. Returns whether the buffers were carved anew (their addresses may have
+// changed even when the arena's base did not).
+bool ensure_wave(rtcuda_scene* s, uint32_t capacity, uint32_t shadow_k, uint32_t max_depth) {
     s->stats_dev.ensure(STAT_TOTAL);
     const size_t k = std::max(1u, shadow_k), n_counters = 4 * ((size_t)max_depth + 3);
-    if (s->arena.base && capacity <= s->arena_capacity && k <= s->arena_shadow_k && max_depth <= s->arena_depth) return;
+    if (s->arena.base && capacity <= s->arena_capacity && k <= s->arena_shadow_k && max_depth <= s->arena_depth) return false;
     const size_t cap = capacity;
     REQUIRE((uint64_t)cap * k < (1ull << 32), "paths in flight x light samples per vertex must stay below 2^32");
     const size_t need = arena_bytes(cap, shadow_k, max_depth);
@@ -1187,9 +1188,54 @@ void ensure_wave(rtcuda_scene* s, uint32_t capacity, uint32_t shadow_k, uint32_t
     view(s->counters, n_counters);
     view(s->counters64, (size_t)max_depth + 3);
     s->arena_capacity = capacity; s->arena_shadow_k = k; s->arena_depth = max_depth;
+    return true;
 }
 
-constexpr size_t MAX_BATCH = (size_t)1 << 28;   // path slots per wavefront batch (see render_device)
+constexpr size_t MAX_BATCH = (size_t)1 << 28;   // path slots per wavefront batch (see batch_shape)
+
+// Batch shape of a wavefront over `n_items` path sources (a frame's pixels, or the live rays of rtcuda_radiance) x `n_samples`
+// samples: items and samples per batch.
+void batch_shape(rtcuda_scene* s, uint32_t n_items, uint32_t n_samples, uint32_t shadow_k, uint32_t max_depth, uint32_t& np_batch,
+                 uint32_t& ns_batch) {
+    // Wavefront size. Deep bounces keep only a fraction of a batch alive (C3: 15 % fewer per bounce, 30 % left at
+    // depth 8) and every launch of a persistent kernel ends with a drain tail, so batches are sized for the 180 GB
+    // of HBM3e, not for L2: up to 256 Mi paths (336 B of path state each with 4 light samples per vertex), capped
+    // to 40 % of the free device memory. C3's 143 M live paths are ONE batch of 111 launches (48 GB); with 64 Mi-path
+    // batches the same frame took 327 launches and 3.4 % longer (profiles/r3a_ab.log).
+    uint32_t capacity = s->ctx->bs.max_paths_in_flight;
+    if (!capacity)
+        if (const char* env = std::getenv("RTCUDA_MAX_PATHS")) capacity = (uint32_t)std::strtoul(env, nullptr, 0);  // tuning aid
+    if (!capacity) {
+        // Memory already held for path state (this scene's arena, or one parked by a released scene) that fits the
+        // wavefront this job wants settles the size without asking the driver: cudaMemGetInfo is a trip into the
+        // kernel driver (it queues behind NVML queries of a monitoring thread and other processes' calls) and sat
+        // inside the render window with the GPU idle — 5-35 ms per frame on a busy box (profiles/r1s_gap.log).
+        const size_t want = std::min<size_t>(MAX_BATCH, std::max<size_t>(1024, (size_t)n_items * n_samples));
+        const size_t held = std::max(s->arena.base ? s->arena.bytes : 0, g_arena_cache.largest(s->ctx->device));
+        if (held >= arena_bytes(want, shadow_k, max_depth)) capacity = (uint32_t)want;
+        else if (held >= ((size_t)8 << 30)) {
+            // a large arena that is smaller than this job's wish was itself cut to the 40 % rule when it was made:
+            // run in batches of what it holds rather than ask the driver again (28 ms in one C5 call, profiles/r4k)
+            const size_t per_slot = arena_bytes(1u << 20, shadow_k, max_depth) >> 20;
+            capacity = (uint32_t)std::min<size_t>(want, (held - (1u << 20)) / std::max<size_t>(1, per_slot));
+        }
+    }
+    if (!capacity) {
+        const size_t bytes_per_slot = 16 + 16 * 7 + 16 + 4 + 48 * (size_t)std::max(1u, shadow_k);
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        const size_t have_b = free_b + s->wave_bytes();
+        capacity = (uint32_t)std::min<size_t>(std::min<size_t>(MAX_BATCH, std::max<size_t>(1024, (size_t)n_items * n_samples)), (size_t)(0.4 * (double)have_b) / bytes_per_slot);
+    }
+    capacity = std::min(capacity, (uint32_t)(0xffffffffull / std::max(1u, shadow_k)));   // shadow-ray queue positions are 32-bit
+    capacity = std::max(capacity, 1024u);
+    np_batch = std::min(n_items, capacity);
+    // samples per batch: as many as fit, then evened out over the batches (256 spp in batches of 124 would end with a
+    // batch of 8 samples, whose launches are all drain tail)
+    ns_batch = std::max(1u, std::min(n_samples, capacity / np_batch));
+    const uint32_t n_sample_batches = (n_samples + ns_batch - 1) / ns_batch;
+    ns_batch = (n_samples + n_sample_batches - 1) / n_sample_batches;
+}
 enum { CLS_EXTEND = 0, CLS_SHADE = 1, CLS_SHADOW = 2, CLS_OTHER = 3, CLS_GATHER = 4, CLS_COUNT = 5 };
 
 // The event pool and the span list are shared by direct launches and by the captured frame (whose event-record nodes keep
@@ -1219,12 +1265,23 @@ struct SpanGuard {  // times one launch when kernel timing is on
     ~SpanGuard() noexcept(false) { if (on) s->spans.push_back({cls, e0, record_event(s)}); }
 };
 
+// The caller's rays of an rtcuda_radiance batch: the chunk's prepared rays, the depth-0 hit k_trace found for each, the stream key
+// of the chunk's first ray, and the call's own launch counter (the scene's counts describe the last render)
+struct CallerRays {
+    const float4* rays;
+    const float4* first_hits;
+    uint32_t key_base;
+    LaunchCounter* lc;
+};
+
 // One batch of the wavefront: raygen, then per bounce extend -> shade -> shadow. All launches are sized by
 // the batch (an upper bound); kernels read the live queue length from device counters, so the host never
-// synchronises inside a batch.
-void run_batch(rtcuda_scene* s, const RenderParams& rp, Wave w, uint32_t n_paths, bool collect) {
+// synchronises inside a batch. With `caller` the paths start from the caller's rays (k_raygen_rays) at their known depth-0 hits:
+// the depth-0 extend is skipped, and no kernel time is recorded.
+void run_batch(rtcuda_scene* s, const RenderParams& rp, Wave w, uint32_t n_paths, bool collect, const CallerRays* caller = nullptr) {
     cudaStream_t st = s->ctx->stream;
-    const bool timing = (s->ctx->bs.collect_stats & RTCUDA_STATS_KERNEL_TIMES) != 0;
+    const bool timing = !caller && (s->ctx->bs.collect_stats & RTCUDA_STATS_KERNEL_TIMES) != 0;
+    LaunchCounter& lc = caller ? *caller->lc : s->lc;
     const uint32_t max_depth = rp.max_ray_depth;
     uint32_t* rays = s->counters.p;                       // rays[d]: queue length at depth d
     uint32_t* fetch_ext = s->counters.p + (max_depth + 3);      // work-fetch cursors of the persistent kernels
@@ -1237,7 +1294,11 @@ void run_batch(rtcuda_scene* s, const RenderParams& rp, Wave w, uint32_t n_paths
     w.ray_o_out = s->ray_o[0].p;
     w.ray_d_out = s->ray_d[0].p;
     w.n_out = rays;
-    { SpanGuard g(s, CLS_OTHER, timing); launch_raygen(st, s->sc, rp, w, n_paths, s->lc); }
+    {
+        SpanGuard g(s, CLS_OTHER, timing);
+        if (caller) launch_raygen_rays(st, rp, w, caller->rays, caller->first_hits, caller->key_base, n_paths, lc);
+        else launch_raygen(st, s->sc, rp, w, n_paths, lc);
+    }
     for (uint32_t depth = 0; depth <= max_depth; depth++) {
         const int in = depth & 1, out = in ^ 1;
         w.depth = depth;
@@ -1245,11 +1306,11 @@ void run_batch(rtcuda_scene* s, const RenderParams& rp, Wave w, uint32_t n_paths
         w.ray_o_out = s->ray_o[out].p; w.ray_d_out = s->ray_d[out].p;
         w.n_in = rays + depth; w.n_out = rays + depth + 1; w.n_shadow = shadows + depth;
         w.deferred = s->deferred.p; w.n_deferred = deferred_n + depth;
-        { SpanGuard g(s, CLS_EXTEND, timing); launch_extend(st, s->sc, w, n_paths, depth == 0 ? s->sc.camera.near_clip : 0.0001f, fetch_ext + depth, collect, s->lc); }
-        { SpanGuard g(s, CLS_SHADE, timing); launch_shade(st, s->sc, rp, w, n_paths, s->lc); }
+        if (depth || !caller) { SpanGuard g(s, CLS_EXTEND, timing); launch_extend(st, s->sc, w, n_paths, depth == 0 ? s->sc.camera.near_clip : 0.0001f, fetch_ext + depth, collect, lc); }
+        { SpanGuard g(s, CLS_SHADE, timing); launch_shade(st, s->sc, rp, w, n_paths, lc); }
         if (depth < max_depth && w.shadow_k) {
-            { SpanGuard g(s, CLS_SHADOW, timing); launch_shadow(st, s->sc, w, (uint32_t)std::min<uint64_t>(0xffffffffull, (uint64_t)n_paths * std::max(1u, w.shadow_k)), fetch_sh + depth, collect, s->lc); }
-            { SpanGuard g(s, CLS_GATHER, timing); launch_shadow_gather(st, w, n_paths, s->lc); }
+            { SpanGuard g(s, CLS_SHADOW, timing); launch_shadow(st, s->sc, w, (uint32_t)std::min<uint64_t>(0xffffffffull, (uint64_t)n_paths * std::max(1u, w.shadow_k)), fetch_sh + depth, collect, lc); }
+            { SpanGuard g(s, CLS_GATHER, timing); launch_shadow_gather(st, w, n_paths, lc); }
         }
     }
 }
@@ -1311,44 +1372,8 @@ void render_device(rtcuda_scene* s, const rtcuda_settings* settings, const rtcud
         if (nb != npix_img && !accumulate) CK(cudaMemsetAsync(out->beauty, 0, npix_img * 12, st));   // (accumulate: the plane holds the running sum)
         if (nb) {
             const uint32_t shadow_k = shadow_entries_per_vertex(s, rp);
-            // Wavefront size. Deep bounces keep only a fraction of a batch alive (C3: 15 % fewer per bounce, 30 % left at
-            // depth 8) and every launch of a persistent kernel ends with a drain tail, so batches are sized for the 180 GB
-            // of HBM3e, not for L2: up to 256 Mi paths (336 B of path state each with 4 light samples per vertex), capped
-            // to 40 % of the free device memory. C3's 143 M live paths are ONE batch of 111 launches (48 GB); with 64 Mi-path
-            // batches the same frame took 327 launches and 3.4 % longer (profiles/r3a_ab.log).
-            uint32_t capacity = s->ctx->bs.max_paths_in_flight;
-            if (!capacity)
-                if (const char* env = std::getenv("RTCUDA_MAX_PATHS")) capacity = (uint32_t)std::strtoul(env, nullptr, 0);  // tuning aid
-            if (!capacity) {
-                // Memory already held for path state (this scene's arena, or one parked by a released scene) that fits the
-                // wavefront this job wants settles the size without asking the driver: cudaMemGetInfo is a trip into the
-                // kernel driver (it queues behind NVML queries of a monitoring thread and other processes' calls) and sat
-                // inside the render window with the GPU idle — 5-35 ms per frame on a busy box (profiles/r1s_gap.log).
-                const size_t want = std::min<size_t>(MAX_BATCH, std::max<size_t>(1024, (size_t)nb * n_samples_total));
-                const size_t held = std::max(s->arena.base ? s->arena.bytes : 0, g_arena_cache.largest(s->ctx->device));
-                if (held >= arena_bytes(want, shadow_k, rp.max_ray_depth)) capacity = (uint32_t)want;
-                else if (held >= ((size_t)8 << 30)) {
-                    // a large arena that is smaller than this job's wish was itself cut to the 40 % rule when it was made:
-                    // run in batches of what it holds rather than ask the driver again (28 ms in one C5 call, profiles/r4k)
-                    const size_t per_slot = arena_bytes(1u << 20, shadow_k, rp.max_ray_depth) >> 20;
-                    capacity = (uint32_t)std::min<size_t>(want, (held - (1u << 20)) / std::max<size_t>(1, per_slot));
-                }
-            }
-            if (!capacity) {
-                const size_t bytes_per_slot = 16 + 16 * 7 + 16 + 4 + 48 * (size_t)std::max(1u, shadow_k);
-                size_t free_b = 0, total_b = 0;
-                CK(cudaMemGetInfo(&free_b, &total_b));
-                const size_t have_b = free_b + s->wave_bytes();
-                capacity = (uint32_t)std::min<size_t>(std::min<size_t>(MAX_BATCH, std::max<size_t>(1024, (size_t)nb * n_samples_total)), (size_t)(0.4 * (double)have_b) / bytes_per_slot);
-            }
-            capacity = std::min(capacity, (uint32_t)(0xffffffffull / std::max(1u, shadow_k)));   // shadow-ray queue positions are 32-bit
-            capacity = std::max(capacity, 1024u);
-            const uint32_t np_batch = std::min(nb, capacity);
-            // samples per batch: as many as fit, then evened out over the batches (256 spp in batches of 124 would end with a
-            // batch of 8 samples, whose launches are all drain tail)
-            uint32_t ns_batch = std::max(1u, std::min(n_samples_total, capacity / np_batch));
-            const uint32_t n_sample_batches = (n_samples_total + ns_batch - 1) / ns_batch;
-            ns_batch = (n_samples_total + n_sample_batches - 1) / n_sample_batches;
+            uint32_t np_batch = 0, ns_batch = 0;
+            batch_shape(s, nb, n_samples_total, shadow_k, rp.max_ray_depth, np_batch, ns_batch);
             tr.mark("sizing");
             ensure_wave(s, np_batch * ns_batch, shadow_k, rp.max_ray_depth);
             s->accum.ensure(nb);
@@ -1642,6 +1667,114 @@ void query_host(rtcuda_scene* s, const QueryPtrs& q, uint64_t count) {
         if (q.ids) CK(cudaMemcpyAsync(q.ids + 2 * b, ids.p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
         if (q.uv) CK(cudaMemcpyAsync(q.uv + 2 * b, uv.p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
         if (q.occluded) CK(cudaMemcpyAsync(q.occluded + b, occ.p, (size_t)n, cudaMemcpyDeviceToHost, st));
+    }
+    CK(cudaStreamSynchronize(st));
+}
+
+// ---------------------------------------------------------------------------------------------------
+// radiance along caller-supplied rays (rtcuda_radiance): the wavefront integrator started from the caller's rays
+// ---------------------------------------------------------------------------------------------------
+// Per chunk of rays: k_radiance_prep normalises them, k_trace walks each first segment once, k_radiance_live lists the rays that
+// need path slots, then batches over (live rays x samples) run the renderer's wavefront from depth 0 with the depth-0 extend
+// skipped, k_resolve sums the samples, and k_finalize writes the means. The call may re-carve the scene's path-state arena; the
+// stats, the launch count and the kernel-time spans of the last render are left alone.
+
+// Checks that need no device: done first, so that a refused call does no device work
+void validate_radiance(const rtcuda_scene* s, const rtcuda_settings* st, const float* rays, uint64_t count, uint32_t stream_base,
+                       const float* radiance) {
+    REQUIRE(count < (1ull << 32), "ray count must be below 2^32");
+    REQUIRE((uint64_t)stream_base + count <= (1ull << 32), "stream_base + count must not exceed 2^32");
+    REQUIRE(rays || count == 0, "rays is NULL");
+    REQUIRE(radiance, "radiance is NULL");
+    REQUIRE(st, "settings is NULL");
+    REQUIRE(st->samples_per_pixel >= 1, "samples_per_pixel must be >= 1");
+    if (st->sampler_kind == RTCUDA_SAMPLER_STRATIFIED) REQUIRE(st->x_strata >= 1 && st->y_strata >= 1, "strata must be >= 1");
+    REQUIRE(s, "scene is NULL");
+}
+
+// Device scratch of one call, sized for its largest chunk
+struct RadianceScratch {
+    DevBuf<float4> prepared, first_hits, accum;
+    DevBuf<uint32_t> live, counters;     // counters: k_trace's fetch cursor, the live-ray count
+    DevBuf<unsigned long long> stats;    // STAT_* of the call's wavefront (the scene's block belongs to the render)
+    LaunchCounter lc;
+    explicit RadianceScratch(uint64_t chunk) {
+        prepared.alloc(2 * chunk); first_hits.alloc(chunk); accum.alloc(chunk); live.alloc(chunk);
+        counters.alloc(2); stats.alloc(STAT_TOTAL);
+    }
+};
+
+// One chunk of n rays: `rays` and `out` are device pointers offset to the chunk, key_base the stream key of its first ray
+void radiance_chunk(rtcuda_scene* s, const rtcuda_settings* settings, const float4* rays, uint32_t n, uint32_t key_base, float* out,
+                    RadianceScratch& x) {
+    cudaStream_t st = s->ctx->stream;
+    RenderParams rp = make_params(settings);
+    rp.antialias_primary_rays = 0;   // a caller's ray has no differentials: its first hit uses matctx_no_aa like every later bounce
+    launch_radiance_prep(st, rays, n, x.prepared.p, x.lc);
+    CK(cudaMemsetAsync(x.counters.p, 0, 2 * sizeof(uint32_t), st));
+    launch_trace(st, s->sc, x.prepared.p, n, x.first_hits.p, x.counters.p, x.lc);
+    launch_radiance_live(st, s->sc, x.prepared.p, x.first_hits.p, n, x.live.p, x.counters.p + 1, x.lc);
+    CK(cudaMemsetAsync(out, 0, (size_t)n * 3 * sizeof(float), st));
+    uint32_t n_live = 0;
+    CK(cudaMemcpyAsync(&n_live, x.counters.p + 1, sizeof n_live, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (!n_live) return;
+    const uint32_t spp = settings->samples_per_pixel, shadow_k = shadow_entries_per_vertex(s, rp);
+    uint32_t np_batch = 0, ns_batch = 0;
+    batch_shape(s, n_live, spp, shadow_k, rp.max_ray_depth, np_batch, ns_batch);
+    // The captured frame graph's nodes hold buffer pointers carved from the arena, and its key holds the arena's base but not the
+    // carve; a re-carve keeps the base when the allocation is big enough (WaveArena::reserve). The graph must not outlive it.
+    if (ensure_wave(s, np_batch * ns_batch, shadow_k, rp.max_ray_depth) && s->frame_exec) {
+        cudaGraphExecDestroy(s->frame_exec);
+        s->frame_exec = nullptr;
+    }
+    CK(cudaMemsetAsync(x.accum.p, 0, (size_t)n_live * sizeof(float4), st));
+    Wave w{};
+    w.pixel_list = x.live.p;
+    w.capacity = np_batch * ns_batch;
+    w.state = s->state.p; w.radiance = s->radiance.p; w.hits = s->hits.p;
+    w.stats = x.stats.p;
+    w.shadow_k = shadow_k; w.svertex = s->svertex.p;
+    w.sray_o = s->sray_o.p; w.sray_d = s->sray_d.p; w.scontrib = s->scontrib.p;
+    const CallerRays caller{x.prepared.p, x.first_hits.p, key_base, &x.lc};
+    for (uint32_t p0 = 0; p0 < n_live; p0 += np_batch) {
+        const uint32_t np = std::min(np_batch, n_live - p0);
+        for (uint32_t s0 = 0; s0 < spp; s0 += ns_batch) {
+            const uint32_t ns = std::min(ns_batch, spp - s0);
+            w.pixel_base = p0; w.n_pixels = np; w.sample_base = s0; w.n_samples = ns;
+            run_batch(s, rp, w, np * ns, false, &caller);
+            launch_resolve(st, w, x.accum.p, x.lc);
+        }
+    }
+    // k_finalize reused with the live list as its pixel list and a width of 65536: idx = (r >> 16) * 65536 + (r & 0xffff) = r,
+    // the ray's index in the chunk (chunks hold at most 2^24 rays)
+    launch_finalize(st, x.live.p, n_live, 65536u, x.accum.p, 1.0f / (float)spp, out, x.stats.p, false, x.lc);
+}
+
+// Device arrays on this scene's GPU; blocks until the radiance is written
+void radiance_device(rtcuda_scene* s, const rtcuda_settings* settings, const float* rays, uint64_t count, uint32_t stream_base, float* radiance) {
+    RadianceScratch x(std::min(count, QUERY_CHUNK));
+    for (uint64_t b = 0; b < count; b += QUERY_CHUNK) {
+        const uint32_t n = (uint32_t)std::min(QUERY_CHUNK, count - b);
+        radiance_chunk(s, settings, (const float4*)rays + 2 * b, n, stream_base + (uint32_t)b, radiance + 3 * b, x);
+    }
+    CK(cudaStreamSynchronize(s->ctx->stream));
+}
+
+// Host arrays: per chunk, rays in and radiance out with cudaMemcpyAsync on the scene's stream; blocks until the radiance is here
+void radiance_host(rtcuda_scene* s, const rtcuda_settings* settings, const float* rays, uint64_t count, uint32_t stream_base, float* radiance) {
+    cudaStream_t st = s->ctx->stream;
+    const uint64_t cap = std::min(count, QUERY_CHUNK);
+    RadianceScratch x(cap);
+    DevBuf<float4> d_rays;
+    DevBuf<float> d_out;
+    d_rays.alloc(2 * cap);
+    d_out.alloc(3 * cap);
+    for (uint64_t b = 0; b < count; b += QUERY_CHUNK) {
+        const uint32_t n = (uint32_t)std::min(QUERY_CHUNK, count - b);
+        CK(cudaMemcpyAsync(d_rays.p, rays + 8 * b, (size_t)n * 32, cudaMemcpyHostToDevice, st));
+        radiance_chunk(s, settings, d_rays.p, n, stream_base + (uint32_t)b, d_out.p, x);
+        CK(cudaMemcpyAsync(radiance + 3 * b, d_out.p, (size_t)n * 12, cudaMemcpyDeviceToHost, st));
     }
     CK(cudaStreamSynchronize(st));
 }
@@ -2100,6 +2233,19 @@ void multi_query_host(rtcuda_scene* parent, const QueryPtrs& q, uint64_t count) 
     });
 }
 
+// Host-array radiance on a multi-device scene: contiguous slices of the rays, one per GPU, each keeping its rays' stream keys
+void multi_radiance_host(rtcuda_scene* parent, const rtcuda_settings* settings, const float* rays, uint64_t count, uint32_t stream_base,
+                         float* radiance) {
+    const size_t n = parent->subs.size();
+    const uint64_t per = (count + n - 1) / n;
+    for_each_device(n, [&](size_t r) {
+        const uint64_t lo = std::min<uint64_t>(count, per * r), hi = std::min<uint64_t>(count, lo + per);
+        if (hi == lo) return;
+        enter(parent->subs[r]);
+        radiance_host(parent->subs[r], settings, rays + 8 * lo, hi - lo, stream_base + (uint32_t)lo, radiance + 3 * lo);
+    });
+}
+
 // rtcuda_get_stats of a multi-device scene: ray / fetch / launch counters summed over the GPUs, times = the slowest GPU
 rtcuda_stats multi_stats(const rtcuda_scene* parent) {
     rtcuda_stats t{};
@@ -2407,6 +2553,34 @@ RTCUDA_API rtcuda_status rtcuda_occluded(rtcuda_scene* scene, const float* rays,
 }
 RTCUDA_API rtcuda_status rtcuda_occluded_device(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded) {
     return query(scene, QueryPtrs{rays, nullptr, nullptr, nullptr, occluded}, count, true);
+}
+
+namespace {
+rtcuda_status radiance_call(rtcuda_scene* scene, const rtcuda_settings* settings, const float* rays, uint64_t count, uint32_t stream_base,
+                            float* radiance, bool device_arrays) {
+    return guarded([&] {
+        validate_radiance(scene, settings, rays, count, stream_base, radiance);
+        if (count == 0) return;
+        if (!device_arrays && !scene->subs.empty()) { multi_radiance_host(scene, settings, rays, count, stream_base, radiance); return; }
+        rtcuda_scene* one = scene->subs.empty() ? scene : scene->subs[0];   // device arrays live on device_ids[0]
+        CK(cudaSetDevice(one->ctx->device));
+        tls_stream = one->ctx->stream;
+        if (!device_arrays) { radiance_host(one, settings, rays, count, stream_base, radiance); return; }
+        REQUIRE(((uintptr_t)rays & 15u) == 0, "rays must be 16-byte aligned");
+        require_device_pointer(rays, one->ctx->device, "rays");
+        require_device_pointer(radiance, one->ctx->device, "radiance");
+        radiance_device(one, settings, rays, count, stream_base, radiance);
+    });
+}
+}  // namespace
+
+RTCUDA_API rtcuda_status rtcuda_radiance(rtcuda_scene* scene, const rtcuda_settings* settings, const float* rays, uint64_t count,
+                                         uint32_t stream_base, float* radiance) {
+    return radiance_call(scene, settings, rays, count, stream_base, radiance, false);
+}
+RTCUDA_API rtcuda_status rtcuda_radiance_device(rtcuda_scene* scene, const rtcuda_settings* settings, const float* rays, uint64_t count,
+                                                uint32_t stream_base, float* radiance) {
+    return radiance_call(scene, settings, rays, count, stream_base, radiance, true);
 }
 
 RTCUDA_API rtcuda_status rtcuda_get_stats(const rtcuda_scene* scene, rtcuda_stats* out) {

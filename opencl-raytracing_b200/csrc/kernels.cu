@@ -92,6 +92,27 @@ __global__ void __launch_bounds__(BLOCK) k_raygen(const __grid_constant__ SceneD
     }
 }
 
+// rtcuda_radiance: k_raygen for caller-supplied rays (rt_query.h raygen_rays_body). Every slot is queued at its own position, so
+// the depth-0 queue length is the batch size.
+__global__ void __launch_bounds__(BLOCK) k_raygen_rays(const __grid_constant__ RenderParams rp, const __grid_constant__ Wave w, const float4* rays,
+                                                        const float4* first_hits, uint32_t key_base, uint32_t n) {
+    const uint32_t i = blockIdx.x * BLOCK + threadIdx.x;
+    if (i == 0) *w.n_out = n;
+    if (i < n) raygen_rays_body(i, rp, w, rays, first_hits, key_base);
+}
+
+// rtcuda_radiance: the indices of a chunk's live rays (rt_query.h radiance_ray_live), one atomic per block like k_raygen
+__global__ void __launch_bounds__(BLOCK) k_radiance_live(const __grid_constant__ SceneD sc, const float4* rays, const float4* first_hits, uint32_t n,
+                                                          uint32_t* live, uint32_t* n_live) {
+    __shared__ uint32_t s_count, s_base;
+    const uint32_t i = blockIdx.x * BLOCK + threadIdx.x;
+    if (threadIdx.x == 0) s_count = 0;
+    __syncthreads();
+    const bool keep = i < n && radiance_ray_live(sc, rays, first_hits, i);
+    const uint32_t pos = block_push(keep, n_live, &s_count, &s_base);
+    if (keep) live[pos] = i;
+}
+
 // Persistent traversal kernels. A warp keeps pulling work from the launch's queue: whenever at least
 // REFILL_MIN lanes are out of work they fetch new rays together (one global atomic per refill), so the walk
 // runs with nearly full warps although the rays of a bounce have wildly different traversal lengths
@@ -422,6 +443,16 @@ __global__ void __launch_bounds__(BLOCK) k_finalize(const uint32_t* pixel_list, 
 
 void launch_raygen(cudaStream_t st, const SceneD& sc, const RenderParams& rp, const Wave& w, uint32_t n, LaunchCounter& lc) {
     k_raygen<<<grid_for(n), BLOCK, 0, st>>>(sc, rp, w, n);
+    lc.launches++;
+}
+void launch_raygen_rays(cudaStream_t st, const RenderParams& rp, const Wave& w, const float4* rays, const float4* first_hits, uint32_t key_base,
+                        uint32_t n, LaunchCounter& lc) {
+    k_raygen_rays<<<grid_for(n), BLOCK, 0, st>>>(rp, w, rays, first_hits, key_base, n);
+    lc.launches++;
+}
+void launch_radiance_live(cudaStream_t st, const SceneD& sc, const float4* rays, const float4* first_hits, uint32_t n, uint32_t* live,
+                          uint32_t* n_live, LaunchCounter& lc) {
+    k_radiance_live<<<grid_for(n), BLOCK, 0, st>>>(sc, rays, first_hits, n, live, n_live);
     lc.launches++;
 }
 static uint32_t persistent_grid(const void* kernel, uint32_t n_max, int block = BLOCK) {

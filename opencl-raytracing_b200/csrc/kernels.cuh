@@ -43,6 +43,14 @@ void launch_occluded(cudaStream_t st, const SceneD& sc, const float4* rays, uint
 void launch_trace_finish(cudaStream_t st, const SceneD& sc, const float4* rays, const float4* hits, uint32_t n, const QueryOut& out,
                          LaunchCounter& lc);
 
+// radiance along caller-supplied rays (rtcuda_radiance, rt_query.h): normalisation (kernels_aov.cu), the live-ray list (`n_live` must
+// be zero), and the depth-0 path slots of a batch, queued with the hits k_trace found
+void launch_radiance_prep(cudaStream_t st, const float4* rays, uint32_t n, float4* prepared, LaunchCounter& lc);
+void launch_radiance_live(cudaStream_t st, const SceneD& sc, const float4* rays, const float4* first_hits, uint32_t n, uint32_t* live,
+                          uint32_t* n_live, LaunchCounter& lc);
+void launch_raygen_rays(cudaStream_t st, const RenderParams& rp, const Wave& w, const float4* rays, const float4* first_hits, uint32_t key_base,
+                        uint32_t n, LaunchCounter& lc);
+
 // BVH build
 void launch_prim_setup(cudaStream_t st, const BuildCtx& b, LaunchCounter& lc);
 void launch_morton(cudaStream_t st, const BuildCtx& b, LaunchCounter& lc);

@@ -60,6 +60,22 @@ void launch_trace_finish(cudaStream_t st, const SceneD& sc, const float4* rays, 
     lc.launches++;
 }
 
+// rtcuda_radiance: the caller's rays normalised (rt_query.h radiance_prep_ray) here, in the IEEE translation unit, so that the CPU
+// reference reproduces the prepared rays bit for bit
+__global__ void __launch_bounds__(BLOCK) k_radiance_prep(const float4* rays, uint32_t n, float4* prepared) {
+    const uint32_t i = blockIdx.x * BLOCK + threadIdx.x;
+    if (i >= n) return;
+    float4 o, d;
+    radiance_prep_ray(rays[2 * (size_t)i], rays[2 * (size_t)i + 1], o, d);
+    prepared[2 * (size_t)i] = o;
+    prepared[2 * (size_t)i + 1] = d;
+}
+
+void launch_radiance_prep(cudaStream_t st, const float4* rays, uint32_t n, float4* prepared, LaunchCounter& lc) {
+    k_radiance_prep<<<grid_for(n), BLOCK, 0, st>>>(rays, n, prepared);
+    lc.launches++;
+}
+
 void launch_aov(cudaStream_t st, const SceneD& sc, const RenderParams& rp, const uint32_t* pixel_list, uint32_t n_pixels,
                 const AovPlanes& planes, unsigned long long* stats, bool collect, LaunchCounter& lc) {
     if (collect) k_aov<true><<<grid_for(n_pixels), BLOCK, 0, st>>>(sc, rp, pixel_list, n_pixels, planes, stats);

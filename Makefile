@@ -7,7 +7,7 @@ HDRS := $(wildcard $(CSRC)/*.h) $(CSRC)/kernels.cuh include/rtcuda.h
 
 all: $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so \
 	tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so tests/hostsim/libhostsim_radiance.so tests/hostsim/liboracle_radiance.so \
-	oracle_ref
+	tests/hostsim/libhostsim_surfaces.so tests/hostsim/liboracle_surfaces.so oracle_ref
 
 # the reference's own C++ device headers compiled for the host (checker of the oracle; no-op when /root/reference is absent)
 .PHONY: oracle_ref
@@ -60,6 +60,16 @@ tests/hostsim/libhostsim_radiance.so: tests/hostsim/hostsim_radiance.cpp tests/h
 tests/hostsim/liboracle_radiance.so: tests/hostsim/oracle_radiance.cpp oracle/oracle.cpp include/rtcuda.h
 	g++ -O2 -std=c++17 -fPIC -ffp-contract=off -fno-fast-math -Wall -Wno-unused-function -pthread -shared -o $@ $<
 
+# the surface query on the CPU (includes hostsim.cpp)
+tests/hostsim/libhostsim_surfaces.so: tests/hostsim/hostsim_surfaces.cpp tests/hostsim/hostsim.cpp $(HDRS)
+	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
+
+# its reference: the oracle's traverse_bvh HitInfo and get_albedo per caller-supplied ray (includes oracle/oracle.cpp, built with the
+# oracle's flags)
+tests/hostsim/liboracle_surfaces.so: tests/hostsim/oracle_surfaces.cpp oracle/oracle.cpp include/rtcuda.h
+	g++ -O2 -std=c++17 -fPIC -ffp-contract=off -fno-fast-math -Wall -Wno-unused-function -pthread -shared -o $@ $<
+
 clean:
 	rm -rf build $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so \
-		tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so tests/hostsim/libhostsim_radiance.so tests/hostsim/liboracle_radiance.so
+		tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so tests/hostsim/libhostsim_radiance.so tests/hostsim/liboracle_radiance.so \
+		tests/hostsim/libhostsim_surfaces.so tests/hostsim/liboracle_surfaces.so

@@ -1,6 +1,8 @@
 #!/usr/bin/env python
 """An equirectangular panorama, a camera the scene format does not have, through CudaRenderer.radiance: one ray per pixel from a
 point inside the Cornell box (longitude across, latitude down, z up), the path tracer's radiance along each, written to EXR.
+CudaRenderer.surfaces on the same rays gives the G-buffer the panorama camera lacks: the shading normal and the albedo at each
+pixel's first hit, written next to it as <out>_normal.exr and <out>_albedo.exr (denoiser guides, for instance).
 
   python examples/panorama.py [out.exr] [width] [spp]    # default panorama.exr, 1024 x 512, 64 spp
 """
@@ -27,5 +29,10 @@ d = np.stack([np.sin(th) * np.cos(ph), np.sin(th) * np.sin(ph), np.cos(th)], axi
 rays = rc.make_rays(eye, d)
 with rc.CudaRenderer(scene) as r:
     radiance = r.radiance(rays, rc.RaytracerSettings(samples_per_pixel=spp)).reshape(H, W, 3)
-exr.write_exr(out_path, {"R": radiance[..., 0], "G": radiance[..., 1], "B": radiance[..., 2]})
-print(f"{out_path}: {W}x{H}, {spp} spp, mean radiance {radiance.mean():.5f}")
+    surf = r.surfaces(rays)
+stem = os.path.splitext(out_path)[0]
+planes = {out_path: radiance, stem + "_normal.exr": surf.normal.reshape(H, W, 3), stem + "_albedo.exr": surf.albedo.reshape(H, W, 3)}
+for path, img in planes.items():
+    exr.write_exr(path, {c: np.ascontiguousarray(img[..., k], np.float32) for k, c in enumerate("RGB")})
+print(f"{out_path}: {W}x{H}, {spp} spp, mean radiance {radiance.mean():.5f}; "
+      f"{stem}_normal.exr, {stem}_albedo.exr: {int((surf.instance != rc._ffi.NONE).sum())} of {W * H} rays hit")

@@ -459,6 +459,42 @@ RTCUDA_API rtcuda_status rtcuda_trace_rays_device(rtcuda_scene* scene, const flo
 RTCUDA_API rtcuda_status rtcuda_occluded(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded);
 RTCUDA_API rtcuda_status rtcuda_occluded_device(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded);
 
+/* One closest hit with the reference's HitInfo (accel.rs:13-25) plus the material's albedo. 64 bytes (four 16-byte
+ * words: the device writes each with one 16-byte store, so device arrays of it must be 16-byte aligned). */
+typedef struct rtcuda_surface {
+    float point[3];  float t;             /* world-space hit point; t exactly as rtcuda_trace_rays reports it */
+    float normal[3]; uint32_t material;   /* HitInfo::normal (world space, unit, NOT flipped toward the ray); instance's material */
+    float uv[2];     uint32_t geom_id; uint32_t prim_id;   /* HitInfo::uv; ids exactly as rtcuda_trace_rays */
+    float albedo[3]; uint32_t light;      /* get_albedo with a zero texture footprint; instance's area light or RTCUDA_NONE */
+} rtcuda_surface;
+
+/* Surface queries: the shading attributes at the closest hit of caller-supplied rays (picking, lightmap and probe set-up, G-buffers
+ * and denoiser guides for cameras the scene format lacks).
+ *   - Rays are packed and accepted exactly like the ray queries above: 8 floats per ray, the same closest-hit rule, the context's
+ *     triangle test, no epsilon, t in units of the direction's length.
+ *   - t, geom_id and prim_id are bit-identical to rtcuda_trace_rays on the same ray (the same walk and object-space re-test).
+ *   - point: o + d * t for triangles; for spheres the object-space hit point taken through the instance's object-to-world transform.
+ *   - normal, uv: the reference's HitInfo::normal / HitInfo::uv, the values of the NORMALS and UV_COORDS first-hit planes. The
+ *     normal is the interpolated vertex normal (or the geometric one of a mesh without normals, or (p - c) / r on a sphere) through
+ *     the instance's inverse transpose, unit length, and not flipped toward the ray. A mesh without uvs uses (0,0), (1,0), (0,1);
+ *     a sphere uses (phi / 2pi, theta / pi).
+ *   - material, light: the hit instance's material index and area light (RTCUDA_NONE when it emits nothing).
+ *   - albedo: the material's albedo with a zero texture footprint (uv only), as the path tracer evaluates every hit that has no ray
+ *     differentials, rtcuda_radiance's first vertex included. A caller's ray has no differentials, so for trilinear (mip-mapped)
+ *     image textures it can differ from the render's ALBEDO plane, which filters over the camera's pixel footprint.
+ *   - Miss, or an invalid ray (the ray-query rule): t = +INFINITY, point / normal / uv / albedo 0, geom_id / prim_id / material /
+ *     light RTCUDA_NONE.
+ *   - rtcuda_trace_surfaces takes HOST arrays and blocks until the records are on the host; on a multi-device scene the rays are cut
+ *     into contiguous slices, one per GPU. rtcuda_trace_surfaces_device takes DEVICE pointers on device_ids[0], rays and surfaces
+ *     16-byte aligned, and blocks until the records are written; the caller must have finished writing the rays.
+ *   - count == 0 is RTCUDA_OK; count >= 2^32, NULL rays with count > 0, NULL surfaces, a NULL scene, or (device variant) a pointer
+ *     that is not device memory of that GPU or is misaligned are RTCUDA_ERR_INVALID_ARGUMENT, refused before any device work.
+ *   - Like the ray queries they read the scene only: rtcuda_get_stats keeps reporting the last render, and nothing a render keeps
+ *     (frame graph, pixel lists, path-state memory) is touched.
+ * Records are the same bit for bit on one GPU, on several, and from host or device arrays. */
+RTCUDA_API rtcuda_status rtcuda_trace_surfaces(rtcuda_scene* scene, const float* rays, uint64_t count, rtcuda_surface* surfaces);
+RTCUDA_API rtcuda_status rtcuda_trace_surfaces_device(rtcuda_scene* scene, const float* rays, uint64_t count, rtcuda_surface* surfaces);
+
 /* Radiance along caller-supplied rays: the path tracer's estimate of the radiance arriving at each ray's origin from its direction
  * (light probes, lightmap texels, cameras the scene format lacks, reference radiance along chosen rays).
  *   - `rays` is `count` x 8 floats per ray, packed like the ray queries: origin.xyz, t_min, direction.xyz, t_max. The direction need

@@ -461,6 +461,21 @@ pub struct RayHit {
     pub barycentrics: [f32; 2],
 }
 
+/// The surface at the closest hit of one query ray (`rtcuda_trace_surfaces`); `light` is the instance's area light or
+/// `RTCUDA_NONE`.
+#[derive(Clone, Copy, Debug, PartialEq)]
+pub struct Surface {
+    pub t: f32,
+    pub point: [f32; 3],
+    pub normal: [f32; 3],
+    pub uv: [f32; 2],
+    pub geom_id: u32,
+    pub prim_id: u32,
+    pub material: u32,
+    pub light: u32,
+    pub albedo: [f32; 3],
+}
+
 impl CudaScene {
     /// Closest hit of every ray in [t_min, t_max] (`[origin.xyz, t_min, direction.xyz, t_max]`): both bounds inclusive, no
     /// back-face culling, equal-t ties to the larger (geom_id, prim_id). The direction is not normalised (t is in its units).
@@ -485,6 +500,22 @@ impl CudaScene {
             check(ffi::rtcuda_occluded(self.scene, rays.as_ptr() as *const f32, rays.len() as u64, occ.as_mut_ptr()), "rtcuda_occluded");
         }
         occ.into_iter().map(|o| o != 0).collect()
+    }
+
+    /// The surface at the closest hit of every ray (`rtcuda_trace_surfaces`, the rule of `trace_rays`): the reference's
+    /// `HitInfo` point, normal (unit, not flipped toward the ray), uv, material and area light, plus the material's albedo with
+    /// a zero texture footprint. A miss is t = +inf, zeros, and `RTCUDA_NONE` ids / material / light.
+    pub fn trace_surfaces(&self, rays: &[[f32; 8]]) -> Vec<Surface> {
+        let mut out = vec![ffi::rtcuda_surface::default(); rays.len()];
+        // SAFETY: [f32; 8] is 8 packed floats; the records are sized for every ray; the call blocks until they are written
+        unsafe {
+            check(ffi::rtcuda_trace_surfaces(self.scene, rays.as_ptr() as *const f32, rays.len() as u64, out.as_mut_ptr()),
+                  "rtcuda_trace_surfaces");
+        }
+        out.iter()
+            .map(|s| Surface { t: s.t, point: s.point, normal: s.normal, uv: s.uv, geom_id: s.geom_id, prim_id: s.prim_id,
+                               material: s.material, light: s.light, albedo: s.albedo })
+            .collect()
     }
 
     /// The path tracer's mean radiance along every ray (`rtcuda_radiance`) over `settings.samples_per_pixel` samples. Directions

@@ -82,6 +82,37 @@ class RayHits:
     barycentrics: np.ndarray   # float32 [N, 2]
 
 
+# one rtcuda_surface record (include/rtcuda.h) as a numpy structured dtype: 64 bytes, the field offsets of _ffi.Surface
+SURFACE_DTYPE = np.dtype([("point", np.float32, (3,)), ("t", np.float32), ("normal", np.float32, (3,)), ("material", np.uint32),
+                          ("uv", np.float32, (2,)), ("geom_id", np.uint32), ("prim_id", np.uint32), ("albedo", np.float32, (3,)),
+                          ("light", np.uint32)])
+
+
+@dataclass
+class RaySurfaces:
+    """The surface at the closest hit of every ray of CudaRenderer.surfaces, one row per ray. t / instance / primitive are those
+    of CudaRenderer.trace; point is the world-space hit point; normal the unit shading normal (interpolated vertex normal, or
+    the geometric one, or the sphere's), not flipped toward the ray; uv the surface's texture coordinates; material and light
+    the instance's material and area light (_ffi.NONE when it emits nothing); albedo the material's albedo at uv with a zero
+    texture footprint. A miss (or an invalid ray) has t = +inf, zeros, and _ffi.NONE ids / material / light. The arrays are views
+    of `records`, one SURFACE_DTYPE record per ray."""
+    records: np.ndarray        # SURFACE_DTYPE [N]
+    t: np.ndarray              # float32 [N]
+    point: np.ndarray          # float32 [N, 3]
+    normal: np.ndarray         # float32 [N, 3]
+    uv: np.ndarray             # float32 [N, 2]
+    instance: np.ndarray       # uint32 [N]
+    primitive: np.ndarray      # uint32 [N]
+    material: np.ndarray       # uint32 [N]
+    light: np.ndarray          # uint32 [N]
+    albedo: np.ndarray         # float32 [N, 3]
+
+    @classmethod
+    def from_records(cls, rec: np.ndarray) -> "RaySurfaces":
+        return cls(rec, rec["t"], rec["point"], rec["normal"], rec["uv"], rec["geom_id"], rec["prim_id"], rec["material"], rec["light"],
+                   rec["albedo"])
+
+
 def _check_rays(rays) -> np.ndarray:
     if not isinstance(rays, np.ndarray) or rays.dtype != np.float32 or rays.ndim != 2 or rays.shape[1] != 8:
         raise ValueError("rays must be a float32 numpy array of shape [N, 8] (see make_rays)")
@@ -237,6 +268,23 @@ class CudaRenderer:
     def occluded_device(self, rays_ptr: int, count: int, occluded_ptr: int) -> None:
         """occluded() on DEVICE arrays (see trace_device): one uint8 per ray, 1 = occluded."""
         _ffi.check(self.lib, self.lib.rtcuda_occluded_device(self._scene, rays_ptr, count, occluded_ptr), "rtcuda_occluded_device")
+
+    def surfaces(self, rays: np.ndarray) -> RaySurfaces:
+        """The surface at the closest hit of every ray of `rays` (float32 [N, 8], make_rays; the rule of trace()): hit point,
+        shading normal, uv, material, area light and albedo (rtcuda_trace_surfaces). Host arrays; blocks until the results are
+        here. Leaves the render state and stats() alone."""
+        rays = _check_rays(rays)
+        rec = np.empty(rays.shape[0], SURFACE_DTYPE)
+        _ffi.check(self.lib, self.lib.rtcuda_trace_surfaces(self._scene, rays.ctypes.data, rays.shape[0], rec.ctypes.data),
+                   "rtcuda_trace_surfaces")
+        return RaySurfaces.from_records(rec)
+
+    def surfaces_device(self, rays_ptr: int, count: int, surfaces_ptr: int) -> None:
+        """surfaces() on DEVICE arrays of the context's first GPU: rays count x 8 float32 and surfaces count x 16 4-byte words
+        (one rtcuda_surface each, e.g. a float32 torch tensor [N, 16] whose integer words 7, 10, 11 and 15 are read through
+        .view(torch.int32)), both 16-byte aligned. Finish writing the rays first (torch.cuda.synchronize()). Blocks until
+        written."""
+        _ffi.check(self.lib, self.lib.rtcuda_trace_surfaces_device(self._scene, rays_ptr, count, surfaces_ptr), "rtcuda_trace_surfaces_device")
 
     def radiance(self, rays: np.ndarray, settings: RaytracerSettings, stream_base: int = 0) -> np.ndarray:
         """float32 [N, 3]: the path tracer's mean radiance along every ray of `rays` (float32 [N, 8], make_rays) over

@@ -7,6 +7,7 @@
 // (crates/raytracing-optix/csrc/host/util.hpp:7-27).
 #include <algorithm>
 #include <chrono>
+#include <cstddef>
 #include <cstdlib>
 #include <cmath>
 #include <cstdio>
@@ -1585,20 +1586,30 @@ void render_pixel(rtcuda_scene* s, const rtcuda_settings* settings, uint32_t x, 
 // the stream-ordered pool, sized for one chunk of rays.
 constexpr uint64_t QUERY_CHUNK = 1ull << 24;   // rays per launch: 512 MB of rays and 256 MB of scratch hits
 
-// Query outputs as the C ABI takes them (occluded set: an occlusion query; otherwise a closest-hit query)
+// Query outputs as the C ABI takes them (occluded set: an occlusion query; surfaces set: a surface query; otherwise a closest-hit
+// query)
 struct QueryPtrs {
     const float* rays;
     float* t;
     uint32_t* ids;
     float* uv;
     uint8_t* occluded;
+    rtcuda_surface* surfaces;
 };
+
+// k_surface_finish writes rtcuda_surface as four float4 (rt_query.h surface_finish_body)
+static_assert(sizeof(rtcuda_surface) == 4 * sizeof(float4), "surface record layout");
+static_assert(offsetof(rtcuda_surface, point) == 0 && offsetof(rtcuda_surface, t) == 12, "surface record layout");
+static_assert(offsetof(rtcuda_surface, normal) == 16 && offsetof(rtcuda_surface, material) == 28, "surface record layout");
+static_assert(offsetof(rtcuda_surface, uv) == 32 && offsetof(rtcuda_surface, geom_id) == 40 && offsetof(rtcuda_surface, prim_id) == 44,
+              "surface record layout");
+static_assert(offsetof(rtcuda_surface, albedo) == 48 && offsetof(rtcuda_surface, light) == 60, "surface record layout");
 
 // Checks that need no device: done first, so that a refused query does no device work
 void validate_query(const rtcuda_scene* s, const QueryPtrs& q, uint64_t count) {
     REQUIRE(count < (1ull << 32), "ray count must be below 2^32");
     REQUIRE(q.rays || count == 0, "rays is NULL");
-    REQUIRE(q.t || q.ids || q.uv || q.occluded, "every output is NULL");
+    REQUIRE(q.t || q.ids || q.uv || q.occluded || q.surfaces, "every output is NULL");
     REQUIRE(s, "scene is NULL");
 }
 
@@ -1621,7 +1632,8 @@ void query_chunk(rtcuda_scene* s, const float4* rays, uint32_t n, const QueryPtr
         return;
     }
     launch_trace(st, s->sc, rays, n, hits, counter, lc);
-    launch_trace_finish(st, s->sc, rays, hits, n, QueryOut{out.t, out.ids, out.uv}, lc);
+    if (out.surfaces) launch_surface_finish(st, s->sc, rays, hits, n, (float4*)out.surfaces, lc);
+    else launch_trace_finish(st, s->sc, rays, hits, n, QueryOut{out.t, out.ids, out.uv}, lc);
 }
 
 // Device arrays on this scene's GPU; blocks until the outputs are written
@@ -1634,7 +1646,7 @@ void query_device(rtcuda_scene* s, const QueryPtrs& q, uint64_t count) {
     for (uint64_t b = 0; b < count; b += QUERY_CHUNK) {
         const uint32_t n = (uint32_t)std::min(QUERY_CHUNK, count - b);
         const QueryPtrs o{nullptr, q.t ? q.t + b : nullptr, q.ids ? q.ids + 2 * b : nullptr, q.uv ? q.uv + 2 * b : nullptr,
-                          q.occluded ? q.occluded + b : nullptr};
+                          q.occluded ? q.occluded + b : nullptr, q.surfaces ? q.surfaces + b : nullptr};
         query_chunk(s, (const float4*)q.rays + 2 * b, n, o, hits.p, counter.p, lc);
     }
     CK(cudaStreamSynchronize(s->ctx->stream));
@@ -1647,7 +1659,7 @@ void query_host(rtcuda_scene* s, const QueryPtrs& q, uint64_t count) {
     LaunchCounter lc;
     const uint64_t cap = std::min(count, QUERY_CHUNK);
     DevBuf<uint32_t> counter;
-    DevBuf<float4> rays, hits;
+    DevBuf<float4> rays, hits, surf;
     DevBuf<float> t, uv;
     DevBuf<uint32_t> ids;
     DevBuf<uint8_t> occ;
@@ -1658,7 +1670,9 @@ void query_host(rtcuda_scene* s, const QueryPtrs& q, uint64_t count) {
     if (q.t) t.alloc(cap);
     if (q.ids) ids.alloc(2 * cap);
     if (q.uv) uv.alloc(2 * cap);
-    const QueryPtrs dev{nullptr, q.t ? t.p : nullptr, q.ids ? ids.p : nullptr, q.uv ? uv.p : nullptr, q.occluded ? occ.p : nullptr};
+    if (q.surfaces) surf.alloc(4 * cap);
+    const QueryPtrs dev{nullptr, q.t ? t.p : nullptr, q.ids ? ids.p : nullptr, q.uv ? uv.p : nullptr, q.occluded ? occ.p : nullptr,
+                        q.surfaces ? (rtcuda_surface*)surf.p : nullptr};
     for (uint64_t b = 0; b < count; b += QUERY_CHUNK) {
         const uint32_t n = (uint32_t)std::min(QUERY_CHUNK, count - b);
         CK(cudaMemcpyAsync(rays.p, q.rays + 8 * b, (size_t)n * 32, cudaMemcpyHostToDevice, st));
@@ -1667,6 +1681,7 @@ void query_host(rtcuda_scene* s, const QueryPtrs& q, uint64_t count) {
         if (q.ids) CK(cudaMemcpyAsync(q.ids + 2 * b, ids.p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
         if (q.uv) CK(cudaMemcpyAsync(q.uv + 2 * b, uv.p, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
         if (q.occluded) CK(cudaMemcpyAsync(q.occluded + b, occ.p, (size_t)n, cudaMemcpyDeviceToHost, st));
+        if (q.surfaces) CK(cudaMemcpyAsync(q.surfaces + b, surf.p, (size_t)n * sizeof(rtcuda_surface), cudaMemcpyDeviceToHost, st));
     }
     CK(cudaStreamSynchronize(st));
 }
@@ -2228,7 +2243,7 @@ void multi_query_host(rtcuda_scene* parent, const QueryPtrs& q, uint64_t count) 
         if (hi == lo) return;
         enter(parent->subs[r]);
         const QueryPtrs slice{q.rays + 8 * lo, q.t ? q.t + lo : nullptr, q.ids ? q.ids + 2 * lo : nullptr, q.uv ? q.uv + 2 * lo : nullptr,
-                              q.occluded ? q.occluded + lo : nullptr};
+                              q.occluded ? q.occluded + lo : nullptr, q.surfaces ? q.surfaces + lo : nullptr};
         query_host(parent->subs[r], slice, hi - lo);
     });
 }
@@ -2531,28 +2546,37 @@ rtcuda_status query(rtcuda_scene* scene, const QueryPtrs& q, uint64_t count, boo
         tls_stream = one->ctx->stream;
         if (!device_arrays) { query_host(one, q, count); return; }
         REQUIRE(((uintptr_t)q.rays & 15u) == 0, "rays must be 16-byte aligned");
+        REQUIRE(((uintptr_t)q.surfaces & 15u) == 0, "surfaces must be 16-byte aligned");
         require_device_pointer(q.rays, one->ctx->device, "rays");
         require_device_pointer(q.t, one->ctx->device, "t");
         require_device_pointer(q.ids, one->ctx->device, "ids");
         require_device_pointer(q.uv, one->ctx->device, "barycentrics");
         require_device_pointer(q.occluded, one->ctx->device, "occluded");
+        require_device_pointer(q.surfaces, one->ctx->device, "surfaces");
         query_device(one, q, count);
     });
 }
 }  // namespace
 
 RTCUDA_API rtcuda_status rtcuda_trace_rays(rtcuda_scene* scene, const float* rays, uint64_t count, float* t, uint32_t* ids, float* barycentrics) {
-    return query(scene, QueryPtrs{rays, t, ids, barycentrics, nullptr}, count, false);
+    return query(scene, QueryPtrs{rays, t, ids, barycentrics, nullptr, nullptr}, count, false);
 }
 RTCUDA_API rtcuda_status rtcuda_trace_rays_device(rtcuda_scene* scene, const float* rays, uint64_t count, float* t, uint32_t* ids,
                                                   float* barycentrics) {
-    return query(scene, QueryPtrs{rays, t, ids, barycentrics, nullptr}, count, true);
+    return query(scene, QueryPtrs{rays, t, ids, barycentrics, nullptr, nullptr}, count, true);
 }
 RTCUDA_API rtcuda_status rtcuda_occluded(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded) {
-    return query(scene, QueryPtrs{rays, nullptr, nullptr, nullptr, occluded}, count, false);
+    return query(scene, QueryPtrs{rays, nullptr, nullptr, nullptr, occluded, nullptr}, count, false);
 }
 RTCUDA_API rtcuda_status rtcuda_occluded_device(rtcuda_scene* scene, const float* rays, uint64_t count, uint8_t* occluded) {
-    return query(scene, QueryPtrs{rays, nullptr, nullptr, nullptr, occluded}, count, true);
+    return query(scene, QueryPtrs{rays, nullptr, nullptr, nullptr, occluded, nullptr}, count, true);
+}
+// (a NULL surfaces pointer is refused as "every output is NULL")
+RTCUDA_API rtcuda_status rtcuda_trace_surfaces(rtcuda_scene* scene, const float* rays, uint64_t count, rtcuda_surface* surfaces) {
+    return query(scene, QueryPtrs{rays, nullptr, nullptr, nullptr, nullptr, surfaces}, count, false);
+}
+RTCUDA_API rtcuda_status rtcuda_trace_surfaces_device(rtcuda_scene* scene, const float* rays, uint64_t count, rtcuda_surface* surfaces) {
+    return query(scene, QueryPtrs{rays, nullptr, nullptr, nullptr, nullptr, surfaces}, count, true);
 }
 
 namespace {

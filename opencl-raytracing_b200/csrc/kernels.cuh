@@ -42,6 +42,9 @@ void launch_occluded(cudaStream_t st, const SceneD& sc, const float4* rays, uint
                      LaunchCounter& lc);
 void launch_trace_finish(cudaStream_t st, const SceneD& sc, const float4* rays, const float4* hits, uint32_t n, const QueryOut& out,
                          LaunchCounter& lc);
+// rtcuda_trace_surfaces: after launch_trace, one thread per ray writes its 64-byte surface record (four float4 at surfaces[4i])
+void launch_surface_finish(cudaStream_t st, const SceneD& sc, const float4* rays, const float4* hits, uint32_t n, float4* surfaces,
+                           LaunchCounter& lc);
 
 // radiance along caller-supplied rays (rtcuda_radiance, rt_query.h): normalisation (kernels_aov.cu), the live-ray list (`n_live` must
 // be zero), and the depth-0 path slots of a batch, queued with the hits k_trace found

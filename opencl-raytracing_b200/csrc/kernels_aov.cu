@@ -60,6 +60,20 @@ void launch_trace_finish(cudaStream_t st, const SceneD& sc, const float4* rays, 
     lc.launches++;
 }
 
+// rtcuda_trace_surfaces, after k_trace: k_trace_finish's ids and re-test, then the hit's HitInfo and albedo, in this translation
+// unit for the same reason (the values of the first-hit NORMALS / UV_COORDS planes)
+__global__ void __launch_bounds__(BLOCK) k_surface_finish(const __grid_constant__ SceneD sc, const float4* rays, const float4* hits, uint32_t n,
+                                                           float4* surfaces) {
+    const uint32_t i = blockIdx.x * BLOCK + threadIdx.x;
+    if (i < n) surface_finish_body(i, sc, rays, hits, surfaces);
+}
+
+void launch_surface_finish(cudaStream_t st, const SceneD& sc, const float4* rays, const float4* hits, uint32_t n, float4* surfaces,
+                           LaunchCounter& lc) {
+    k_surface_finish<<<grid_for(n), BLOCK, 0, st>>>(sc, rays, hits, n, surfaces);
+    lc.launches++;
+}
+
 // rtcuda_radiance: the caller's rays normalised (rt_query.h radiance_prep_ray) here, in the IEEE translation unit, so that the CPU
 // reference reproduces the prepared rays bit for bit
 __global__ void __launch_bounds__(BLOCK) k_radiance_prep(const float4* rays, uint32_t n, float4* prepared) {

@@ -1,6 +1,7 @@
 // rt_query.h — ray queries on an uploaded scene (rtcuda_trace_rays / rtcuda_occluded): the per-ray logic of k_trace (kernels.cu,
 // the traversal) and k_trace_finish (kernels_aov.cu, ids and the object-space re-test), shared with the CPU harness. Also the
-// per-ray stages of rtcuda_radiance (prep, live list, ray generation) that feed the caller's rays into the wavefront integrator.
+// surface record of rtcuda_trace_surfaces (k_surface_finish, kernels_aov.cu), and the per-ray stages of rtcuda_radiance (prep,
+// live list, ray generation) that feed the caller's rays into the wavefront integrator.
 //
 // A query ray is two float4, (origin.xyz, t_min) and (direction.xyz, t_max): the shape of the wavefront's ray queue. Closest hit
 // and occlusion follow the acceptance rule of the extend / shadow walks (rt_traverse.h): hits with t in [t_min, t_max], both
@@ -63,6 +64,41 @@ RT_HD void trace_finish_body(uint32_t i, const SceneD& sc, const float4* rays, c
     if (out.t) out.t[i] = h.t;
     if (out.ids) { out.ids[2 * (size_t)i] = geom; out.ids[2 * (size_t)i + 1] = pid; }
     if (out.uv) { out.uv[2 * (size_t)i] = h.u; out.uv[2 * (size_t)i + 1] = h.v; }
+}
+
+// ---- the surface at caller-supplied rays' closest hits (rtcuda_trace_surfaces) ------------------------------------------------
+// Ray i's record is four float4 at out[4i]: the layout of rtcuda_surface (include/rtcuda.h; api.cu static_asserts it):
+//   (point.xyz, t), (normal.xyz, material), (uv.xy, geom_id, prim_id), (albedo.xyz, light).
+// t and the ids are trace_finish_body's (ids from the primitive slot, the winner re-tested in object space over the ray's own range);
+// point / normal / uv / material / light are reconstruct_hit's HitInfo, and the albedo is get_albedo with a zero texture footprint,
+// as for every hit without ray differentials. A miss (or an invalid ray, which k_trace misses) is (0, +inf), (0, NONE),
+// (0, 0, NONE, NONE), (0, NONE).
+RT_HD void surface_finish_body(uint32_t i, const SceneD& sc, const float4* rays, const float4* hits, float4* out) {
+    const float4 e = hits[i];
+    Hit h;
+    h.t = e.x; h.prim = f2u(e.y); h.u = e.z; h.v = e.w;
+    float4* o = out + 4 * (size_t)i;
+    if (h.prim == NONE) {
+        o[0] = make_float4(0.0f, 0.0f, 0.0f, RT_INF);
+        o[1] = make_float4(0.0f, 0.0f, 0.0f, u2f(NONE));
+        o[2] = make_float4(0.0f, 0.0f, u2f(NONE), u2f(NONE));
+        o[3] = make_float4(0.0f, 0.0f, 0.0f, u2f(NONE));
+        return;
+    }
+    const Prim* pr = sc.prims + h.prim;
+    const uint32_t geom = f2u(ldg(&pr->a).w), pid = f2u(ldg(&pr->b).w);
+    const float4 o4 = rays[2 * (size_t)i], d4 = rays[2 * (size_t)i + 1];
+    Ray ray;
+    ray.o = xyz(o4);
+    ray.d = xyz(d4);
+    refine_triangle_hit_in_object_space(sc, ray, o4.w, d4.w, h);
+    HitInfo hit;
+    reconstruct_hit(sc, ray.o, ray.d, h, false, hit);
+    const V3 a = get_albedo(sc, sc.materials[hit.material], matctx_no_aa(hit.uv));
+    o[0] = make_float4(hit.point.x, hit.point.y, hit.point.z, h.t);
+    o[1] = make_float4(hit.normal.x, hit.normal.y, hit.normal.z, u2f(hit.material));
+    o[2] = make_float4(hit.uv.x, hit.uv.y, u2f(geom), u2f(pid));
+    o[3] = make_float4(a.x, a.y, a.z, u2f(hit.light));
 }
 
 // ---- radiance along caller-supplied rays (rtcuda_radiance) -------------------------------------------------------------------

@@ -5,9 +5,7 @@ CSRC := $(PKG)/csrc
 NVCCFLAGS := -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -Xcompiler -fvisibility=hidden $(NVCCFLAGS_EXTRA)
 HDRS := $(wildcard $(CSRC)/*.h) $(CSRC)/kernels.cuh include/rtcuda.h
 
-all: $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so \
-	tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so tests/hostsim/libhostsim_radiance.so tests/hostsim/liboracle_radiance.so \
-	tests/hostsim/libhostsim_surfaces.so tests/hostsim/liboracle_surfaces.so oracle_ref
+all: $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so oracle_ref
 
 # the reference's own C++ device headers compiled for the host (checker of the oracle; no-op when /root/reference is absent)
 .PHONY: oracle_ref
@@ -34,42 +32,12 @@ build/api.o: $(CSRC)/api.cu $(HDRS)
 $(PKG)/libraytracing_cuda.so: build/kernels.o build/kernels_aov.o build/api.o
 	$(NVCC) -shared -o $@ $^ -lcudart_static -lrt -lpthread -ldl
 
-oracle/liboracle.so: oracle/oracle.cpp include/rtcuda.h
+oracle/liboracle.so: oracle/rays.cpp oracle/oracle.cpp include/rtcuda.h
 	$(MAKE) -C oracle liboracle.so
 
-tests/hostsim/libhostsim.so: tests/hostsim/hostsim.cpp $(HDRS)
+# the CPU harness: a library is one translation unit of the same name (libhostsim.so: every entry point of hostsim.cpp)
+tests/hostsim/lib%.so: tests/hostsim/%.cpp $(HDRS)
 	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
-
-# the scene-update refit on the CPU (includes hostsim.cpp)
-tests/hostsim/libhostsim_update.so: tests/hostsim/hostsim_update.cpp tests/hostsim/hostsim.cpp $(HDRS)
-	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
-
-# the ray queries on the CPU (includes hostsim.cpp)
-tests/hostsim/libhostsim_query.so: tests/hostsim/hostsim_query.cpp tests/hostsim/hostsim.cpp $(HDRS)
-	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
-
-# their reference: the oracle's traverse_bvh per caller-supplied ray (includes oracle/oracle.cpp, built with the oracle's flags)
-tests/hostsim/liboracle_query.so: tests/hostsim/oracle_query.cpp oracle/oracle.cpp include/rtcuda.h
-	g++ -O2 -std=c++17 -fPIC -ffp-contract=off -fno-fast-math -Wall -Wno-unused-function -pthread -shared -o $@ $<
-
-# radiance along caller-supplied rays on the CPU (includes hostsim.cpp)
-tests/hostsim/libhostsim_radiance.so: tests/hostsim/hostsim_radiance.cpp tests/hostsim/hostsim.cpp $(HDRS)
-	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
-
-# its reference: the oracle's ray_radiance per caller-supplied ray (includes oracle/oracle.cpp, built with the oracle's flags)
-tests/hostsim/liboracle_radiance.so: tests/hostsim/oracle_radiance.cpp oracle/oracle.cpp include/rtcuda.h
-	g++ -O2 -std=c++17 -fPIC -ffp-contract=off -fno-fast-math -Wall -Wno-unused-function -pthread -shared -o $@ $<
-
-# the surface query on the CPU (includes hostsim.cpp)
-tests/hostsim/libhostsim_surfaces.so: tests/hostsim/hostsim_surfaces.cpp tests/hostsim/hostsim.cpp $(HDRS)
-	g++ -O2 -std=c++17 -fPIC -shared -pthread -o $@ $<
-
-# its reference: the oracle's traverse_bvh HitInfo and get_albedo per caller-supplied ray (includes oracle/oracle.cpp, built with the
-# oracle's flags)
-tests/hostsim/liboracle_surfaces.so: tests/hostsim/oracle_surfaces.cpp oracle/oracle.cpp include/rtcuda.h
-	g++ -O2 -std=c++17 -fPIC -ffp-contract=off -fno-fast-math -Wall -Wno-unused-function -pthread -shared -o $@ $<
 
 clean:
-	rm -rf build $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so tests/hostsim/libhostsim_update.so \
-		tests/hostsim/libhostsim_query.so tests/hostsim/liboracle_query.so tests/hostsim/libhostsim_radiance.so tests/hostsim/liboracle_radiance.so \
-		tests/hostsim/libhostsim_surfaces.so tests/hostsim/liboracle_surfaces.so
+	rm -rf build $(PKG)/libraytracing_cuda.so oracle/liboracle.so tests/hostsim/libhostsim.so

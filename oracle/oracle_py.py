@@ -27,9 +27,9 @@ class OracleStats(C.Structure):
 
 
 def build(force: bool = False) -> str:
-    src = os.path.join(_HERE, "oracle.cpp")
-    hdr = os.path.join(os.path.dirname(_HERE), "include", "rtcuda.h")
-    if force or not os.path.exists(LIB_PATH) or os.path.getmtime(LIB_PATH) < max(os.path.getmtime(src), os.path.getmtime(hdr)):
+    """make the library when it is missing or older than a source it compiles (oracle/Makefile holds the flags)"""
+    srcs = [os.path.join(_HERE, f) for f in ("rays.cpp", "oracle.cpp")] + [os.path.join(os.path.dirname(_HERE), "include", "rtcuda.h")]
+    if force or not os.path.exists(LIB_PATH) or os.path.getmtime(LIB_PATH) < max(os.path.getmtime(s) for s in srcs):
         subprocess.check_call(["make", "-C", _HERE, "-B", "liboracle.so"], stdout=subprocess.DEVNULL)
     return LIB_PATH
 
@@ -62,7 +62,7 @@ def use_native_build() -> str:
 def lib() -> C.CDLL:
     global _lib
     if _lib is None:
-        if _lib_path == LIB_PATH and not os.path.exists(LIB_PATH):
+        if _lib_path == LIB_PATH:
             build()
         l = C.CDLL(_lib_path)
         l.oracle_render.argtypes = [C.POINTER(_ffi.SceneDesc), C.POINTER(_ffi.Settings), C.POINTER(_ffi.Outputs), C.c_uint32,
@@ -128,3 +128,52 @@ def render_pixel(scene, settings, x, y, lo, hi, brute_force: bool = False):
     if lib().oracle_render_pixel(C.byref(holder.desc), C.byref(s), x, y, lo, hi, buf, FLAG_BRUTE_FORCE if brute_force else 0) != 0:
         raise RuntimeError("oracle_render_pixel failed")
     return [rc.SinglePixelOutput(b.sample_index, bool(b.hit), tuple(b.uv), tuple(b.normal), tuple(b.radiance)) for b in buf[:n]]
+
+
+def _ray_fn(name: str, argtypes):
+    """an entry point of rays.cpp, which the CPU-baseline build of use_native_build() (oracle.cpp alone) does not hold"""
+    fn = getattr(lib(), name)
+    fn.argtypes, fn.restype = argtypes, C.c_int
+    return fn
+
+
+def trace_rays(scene, rays, brute_force: bool = False):
+    """oracle_trace_rays: traverse_bvh per packed ray [N, 8] over the oracle's BVH2 (or every primitive in build order) ->
+    (t [N] float32, ids [N, 2] uint32, barycentrics [N, 2] float32, occluded [N] uint8)"""
+    rays = np.ascontiguousarray(rays, dtype=np.float32)
+    n = rays.shape[0]
+    holder = scene.to_desc()
+    t, ids, uv, occ = np.empty(n, np.float32), np.empty((n, 2), np.uint32), np.empty((n, 2), np.float32), np.empty(n, np.uint8)
+    fn = _ray_fn("oracle_trace_rays", [C.POINTER(_ffi.SceneDesc), C.c_void_p, C.c_uint64, C.c_uint32] + [C.c_void_p] * 4)
+    if fn(C.byref(holder.desc), rays.ctypes.data, n, FLAG_BRUTE_FORCE if brute_force else 0, t.ctypes.data, ids.ctypes.data,
+          uv.ctypes.data, occ.ctypes.data) != 0:
+        raise RuntimeError("oracle_trace_rays failed")
+    return t, ids, uv, occ
+
+
+def trace_surfaces(scene, rays, brute_force: bool = False):
+    """oracle_trace_surfaces: traverse_bvh's HitInfo per packed ray [N, 8] over the oracle's BVH2 (or every primitive in build
+    order) and get_albedo with a zero footprint -> one rtcuda_surface record per ray (raytracing_cuda.backend.SURFACE_DTYPE [N])"""
+    from raytracing_cuda.backend import SURFACE_DTYPE
+    rays = np.ascontiguousarray(rays, dtype=np.float32)
+    holder = scene.to_desc()
+    rec = np.empty(rays.shape[0], SURFACE_DTYPE)
+    fn = _ray_fn("oracle_trace_surfaces", [C.POINTER(_ffi.SceneDesc), C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p])
+    if fn(C.byref(holder.desc), rays.ctypes.data, rays.shape[0], FLAG_BRUTE_FORCE if brute_force else 0, rec.ctypes.data) != 0:
+        raise RuntimeError("oracle_trace_surfaces failed")
+    return rec
+
+
+def radiance(scene, settings, rays, stream_base: int = 0, num_threads: int = 8):
+    """oracle_radiance: ray_radiance per packed ray [N, 8] and sample over the ray's normalised range -> (radiance [N, 3]
+    float32, prepared rays [N, 8] float32)"""
+    rays = np.ascontiguousarray(rays, dtype=np.float32)
+    n = rays.shape[0]
+    holder = scene.to_desc()
+    s = settings.to_c()
+    out, prep = np.empty((n, 3), np.float32), np.empty((n, 8), np.float32)
+    fn = _ray_fn("oracle_radiance", [C.POINTER(_ffi.SceneDesc), C.POINTER(_ffi.Settings), C.c_void_p, C.c_uint64, C.c_uint32,
+                                     C.c_uint32, C.c_void_p, C.c_void_p])
+    if fn(C.byref(holder.desc), C.byref(s), rays.ctypes.data, n, stream_base, num_threads, out.ctypes.data, prep.ctypes.data) != 0:
+        raise RuntimeError("oracle_radiance failed")
+    return out, prep

@@ -41,22 +41,15 @@ SCENES = {
 }
 
 
-@pytest.fixture(scope="module")
-def hr():
-    import hostsim_radiance_py
-    hostsim_radiance_py.build()
-    return hostsim_radiance_py
-
-
 @pytest.mark.parametrize("name", sorted(SCENES))
-def test_radiance_matches_the_reference(rc, hr, name):
+def test_radiance_matches_the_reference(rc, oracle, name):
     make, seed, gates = SCENES[name]
     sc = make(rc)
     rays, invalid = query_rays(sc, n=1 << 14, seed=seed)
     st = rc.RaytracerSettings(**SETTINGS)
     with rc.CudaRenderer(sc) as r:
         got = r.radiance(rays, st)
-    ref, _ = hr.oracle_radiance(sc, st, rays)
+    ref, _ = oracle.radiance(sc, st, rays)
     assert got.shape == (len(rays), 3) and got.dtype == np.float32
     assert not got[invalid].any()
     if gates is None:

@@ -37,21 +37,14 @@ SCENES = {
 }
 
 
-@pytest.fixture(scope="module")
-def hq():
-    import hostsim_query_py
-    hostsim_query_py.build()
-    return hostsim_query_py
-
-
 @pytest.mark.parametrize("name,watertight", [("C2", False), ("C3", False), ("sphere_scene", False), ("C3", True)])
-def test_queries_match_the_reference(rc, hq, name, watertight):
+def test_queries_match_the_reference(rc, oracle, name, watertight):
     make, brute, seed = SCENES[name]
     sc = make(rc)
     rays, degenerate = query_rays(sc, seed=seed)
     with rc.CudaRenderer(sc, rc.CudaBackendSettings(watertight=watertight)) as r:
         got = _trace(r, rays)
-    rep = compare(got, hq.oracle_trace_rays(sc, rays, brute_force=brute))
+    rep = compare(got, oracle.trace_rays(sc, rays, brute_force=brute))
     print(name, "watertight" if watertight else "", rep)
     assert rep["hit_rays"] > rep["rays"] // 3
     assert rep["id_agreement"] >= ID_AGREEMENT, rep

@@ -1,5 +1,5 @@
 """The ray-query bodies of the CUDA library (rt_query.h: the traversal k_trace runs, then the k_trace_finish body) on the CPU,
-against the reference: the oracle's traverse_bvh per ray over the ray's own [t_min, t_max] (tests/hostsim/oracle_query.cpp),
+against the reference: the oracle's traverse_bvh per ray over the ray's own [t_min, t_max] (oracle_trace_rays in oracle/rays.cpp),
 brute force on the small scenes, over the oracle's BVH2 on the bunny scenes.
 
 Measured (2^16 seeded rays per scene, tests/ray_sets.py): with Moller-Trumbore on cb, the sphere scene,
@@ -23,13 +23,6 @@ SCENES = {
 }
 
 
-@pytest.fixture(scope="module")
-def hq():
-    import hostsim_query_py
-    hostsim_query_py.build()
-    return hostsim_query_py
-
-
 def _check(got, ref, degenerate, outlier_gate):
     rep = compare(got, ref)
     assert rep["hit_rays"] > rep["rays"] // 3, rep
@@ -43,30 +36,30 @@ def _check(got, ref, degenerate, outlier_gate):
 
 
 @pytest.mark.parametrize("name", sorted(SCENES))
-def test_queries_match_the_reference(rc, hq, name):
+def test_queries_match_the_reference(rc, hostsim, oracle, name):
     make, brute, seed = SCENES[name]
     sc = make(rc)
     rays, degenerate = query_rays(sc, seed=seed)
-    _check(hq.trace_rays(sc, rays), hq.oracle_trace_rays(sc, rays, brute_force=brute), degenerate, 0.0)
+    _check(hostsim.trace_rays(sc, rays), oracle.trace_rays(sc, rays, brute_force=brute), degenerate, 0.0)
 
 
-def test_watertight_queries_match_the_reference(rc, hq, monkeypatch):
+def test_watertight_queries_match_the_reference(rc, hostsim, oracle, monkeypatch):
     monkeypatch.setenv("HOSTSIM_WATERTIGHT", "1")
     sc = load_scene("cbbunny_area_light_transforms", 64, 64)
     rays, degenerate = query_rays(sc, seed=5)
-    _check(hq.trace_rays(sc, rays), hq.oracle_trace_rays(sc, rays), degenerate, 6.7e-4)
+    _check(hostsim.trace_rays(sc, rays), oracle.trace_rays(sc, rays), degenerate, 6.7e-4)
 
 
-def test_misses_and_ranges(rc, hq):
+def test_misses_and_ranges(rc, hostsim):
     """a miss is (inf, NONE, NONE, 0, 0); t_max below the hit's t misses, t_min = t_max = t hits (inclusive bounds)"""
     import numpy as np
     sc = load_scene("cb", 64, 64)
     rays = rc.make_rays([[0.0, 0.0, 0.75]] * 4, [[0.0, 0.0, -1.0], [0.0, 0.0, -1.0], [0.0, 0.0, -1.0], [0.0, 0.0, 0.0]])
-    t, ids, uv, occ = hq.trace_rays(sc, rays[:1])
+    t, ids, uv, occ = hostsim.trace_rays(sc, rays[:1])
     assert ids[0, 0] != NONE and t[0] > 0
     rays[1, 7] = np.nextafter(t[0], np.float32(0))
     rays[2, 3] = rays[2, 7] = t[0]
-    t2, ids2, uv2, occ2 = hq.trace_rays(sc, rays)
+    t2, ids2, uv2, occ2 = hostsim.trace_rays(sc, rays)
     assert t2[1] == np.inf and (ids2[1] == NONE).all() and (uv2[1] == 0).all() and occ2[1] == 0
     assert t2[2] == t[0] and (ids2[2] == ids[0]).all() and occ2[2] == 1
     assert t2[3] == np.inf and (ids2[3] == NONE).all() and occ2[3] == 0

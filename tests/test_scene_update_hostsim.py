@@ -10,13 +10,6 @@ from conftest import load_scene
 from scene_motion import about, moved, trs
 
 
-@pytest.fixture(scope="module")
-def hsu():
-    import hostsim_update_py
-    hostsim_update_py.build()
-    return hostsim_update_py
-
-
 def _bits(a):
     """float32 words as u32, with -0.0 read as +0.0 (the only difference min / max of equal boxes can make: fminf(-0, +0)
     may return either, and the refit unions a leaf's boxes in slot order where the build merged them in tree order)"""
@@ -54,8 +47,8 @@ def _assert_same_frame(a, b):
 
 
 @pytest.mark.parametrize("name", ["cb", "cbbunny_area_light_transforms", "sphere"])
-def test_refit_with_unchanged_transforms_reproduces_the_tree(rc, hsu, name):
-    nodes_b, nodes_r, prims_b, prims_r, (sah_b, sah_r) = hsu.refit_identity(_scene(rc, name))
+def test_refit_with_unchanged_transforms_reproduces_the_tree(rc, hostsim, name):
+    nodes_b, nodes_r, prims_b, prims_r, (sah_b, sah_r) = hostsim.refit_identity(_scene(rc, name))
     assert len(nodes_b) and len(prims_b)
     assert np.array_equal(_bits(prims_b), _bits(prims_r))
     assert np.array_equal(_bits(nodes_b), _bits(nodes_r))
@@ -75,14 +68,13 @@ MOTIONS = {
 
 
 @pytest.mark.parametrize("motion", sorted(MOTIONS))
-def test_refit_renders_the_frame_of_a_fresh_build(rc, hostsim, hsu, motion):
+def test_refit_renders_the_frame_of_a_fresh_build(rc, hostsim, motion):
     name, move = MOTIONS[motion]
     a = _scene(rc, name)
     b = move(a)
     st = _settings(rc)
     fresh, _ = hostsim.render(b, st)
-    _assert_same_frame(hsu.render(b, st)[0], fresh)   # the update harness renders like the harness
-    upd, _, (last, sah) = hsu.update_render(a, b, st)
+    upd, _, (last, sah) = hostsim.update_render(a, b, st)
     assert last == 2 and sah > 1.0
     _assert_same_frame(upd, fresh)
     if motion != "moved_camera" and "light" not in motion:   # the instance moved on screen
@@ -90,14 +82,13 @@ def test_refit_renders_the_frame_of_a_fresh_build(rc, hostsim, hsu, motion):
 
 
 @pytest.mark.parametrize("motion", ["translated_instance", "moved_sphere", "moved_area_light"])
-def test_rebuild_renders_the_frame_of_a_fresh_build(rc, hostsim, hsu, motion):
+def test_rebuild_renders_the_frame_of_a_fresh_build(rc, hostsim, motion):
     name, move = MOTIONS[motion]
     a = _scene(rc, name)
     b = move(a)
     st = _settings(rc)
-    fresh, _ = hostsim.render(b, st)
-    upd, us, (last, sah) = hsu.update_render(a, b, st, max_growth=0.0)   # the rule then always asks for the rebuild
+    fresh, fs = hostsim.render(b, st)
+    upd, us, (last, sah) = hostsim.update_render(a, b, st, max_growth=0.0)   # the rule then always asks for the rebuild
     assert last == 3 and sah > 1.0
     _assert_same_frame(upd, fresh)
-    fs = hsu.render(b, st)[1]
     assert (us["nodes_fetched"], us["prims_fetched"]) == (fs["nodes_fetched"], fs["prims_fetched"])   # the same tree as a fresh build

@@ -31,22 +31,15 @@ SCENES = {
 }
 
 
-@pytest.fixture(scope="module")
-def hs():
-    import hostsim_surfaces_py
-    hostsim_surfaces_py.build()
-    return hostsim_surfaces_py
-
-
 @pytest.mark.parametrize("name,watertight", [("C2", False), ("C3", False), ("sphere_scene", False), ("texture_zoo", False), ("C3", True)])
-def test_surfaces_match_the_reference(rc, hs, name, watertight):
+def test_surfaces_match_the_reference(rc, oracle, name, watertight):
     make, brute, seed = SCENES[name]
     sc = make(rc)
     rays, invalid = query_rays(sc, seed=seed)
     with rc.CudaRenderer(sc, rc.CudaBackendSettings(watertight=watertight)) as r:
         got = r.surfaces(rays).records
         h = r.trace(rays)
-    rep = compare_surfaces(got, hs.oracle_trace_surfaces(sc, rays, brute_force=brute))
+    rep = compare_surfaces(got, oracle.trace_surfaces(sc, rays, brute_force=brute))
     print(name, "watertight" if watertight else "", rep)
     assert rep["hit_rays"] > rep["rays"] // 3
     assert rep["id_agreement"] >= ID_AGREEMENT, rep

@@ -1,8 +1,8 @@
 """The surface-query body of the CUDA library (rt_query.h: the traversal k_trace runs, then the k_surface_finish body) on the CPU,
 against the reference: the oracle's traverse_bvh per ray over the ray's own [t_min, t_max] and the winner's HitInfo (point,
-normal, uv, material, light) with get_albedo at a zero footprint (tests/hostsim/oracle_surfaces.cpp), brute force on the small
-scenes, over the oracle's BVH2 on the bunny scenes. The harness (tests/hostsim/hostsim_surfaces.cpp) and the closest-hit harness
-(tests/hostsim/hostsim_query.cpp) build the same scene the same way, so their t and ids can be compared bit for bit.
+normal, uv, material, light) with get_albedo at a zero footprint (oracle_trace_surfaces in oracle/rays.cpp), brute force on
+the small scenes, over the oracle's BVH2 on the bunny scenes. The harness's surface and closest-hit queries
+(tests/hostsim/hostsim.cpp) build the same scene the same way, so their t and ids can be compared bit for bit.
 
 Measured (2^16 seeded rays per scene, tests/ray_sets.py): on cb, the sphere scene, cbbunny_area_light_transforms (C3), the
 reused-mesh scene (normals through rotations and non-uniform scales), the texture zoo (every texture kind, format, wrap mode and
@@ -29,23 +29,9 @@ SCENES = {
 }
 
 
-@pytest.fixture(scope="module")
-def hs():
-    import hostsim_surfaces_py
-    hostsim_surfaces_py.build()
-    return hostsim_surfaces_py
-
-
-@pytest.fixture(scope="module")
-def hq():
-    import hostsim_query_py
-    hostsim_query_py.build()
-    return hostsim_query_py
-
-
-def _check(hs, hq, sc, rays, invalid, brute, outlier_gate):
-    got = hs.trace_surfaces(sc, rays)
-    ref = hs.oracle_trace_surfaces(sc, rays, brute_force=brute)
+def _check(hostsim, oracle, sc, rays, invalid, brute, outlier_gate):
+    got = hostsim.trace_surfaces(sc, rays)
+    ref = oracle.trace_surfaces(sc, rays, brute_force=brute)
     rep = compare_surfaces(got, ref)
     print(rep)
     assert rep["hit_rays"] > rep["rays"] // 3, rep
@@ -54,7 +40,7 @@ def _check(hs, hq, sc, rays, invalid, brute, outlier_gate):
     assert rep["material_light_mismatches"] == 0, rep
     assert is_miss_record(got[invalid]).all() and is_miss_record(ref[invalid]).all()
     # t and the ids are those of the closest-hit query, bit for bit
-    t, ids, _, _ = hq.trace_rays(sc, rays)
+    t, ids, _, _ = hostsim.trace_rays(sc, rays)
     assert np.array_equal(got["t"].view(np.uint32), t.view(np.uint32))
     assert np.array_equal(got["geom_id"], ids[:, 0]) and np.array_equal(got["prim_id"], ids[:, 1])
     # a miss of the closest-hit query is the miss record
@@ -63,26 +49,26 @@ def _check(hs, hq, sc, rays, invalid, brute, outlier_gate):
 
 
 @pytest.mark.parametrize("name", sorted(SCENES))
-def test_surfaces_match_the_reference(rc, hs, hq, name):
+def test_surfaces_match_the_reference(rc, hostsim, oracle, name):
     make, brute, seed = SCENES[name]
     sc = make(rc)
     rays, invalid = query_rays(sc, seed=seed)
-    _check(hs, hq, sc, rays, invalid, brute, 0.0)
+    _check(hostsim, oracle, sc, rays, invalid, brute, 0.0)
 
 
-def test_watertight_surfaces_match_the_reference(rc, hs, hq, monkeypatch):
+def test_watertight_surfaces_match_the_reference(rc, hostsim, oracle, monkeypatch):
     monkeypatch.setenv("HOSTSIM_WATERTIGHT", "1")
     sc = load_scene("cbbunny_area_light_transforms", 64, 64)
     rays, invalid = query_rays(sc, seed=7)
-    _check(hs, hq, sc, rays, invalid, False, 2e-4)
+    _check(hostsim, oracle, sc, rays, invalid, False, 2e-4)
 
 
-def test_surface_fields(rc, hs):
+def test_surface_fields(rc, hostsim):
     """what a caller relies on without a reference: unit normals, the point on the ray at t for triangles, the instance's
     material and light"""
     sc = load_scene("cbbunny_area_light_transforms", 64, 64)
     rays, _ = query_rays(sc, seed=8)
-    got = hs.trace_surfaces(sc, rays)
+    got = hostsim.trace_surfaces(sc, rays)
     hit = got["geom_id"] != 0xFFFFFFFF
     np.testing.assert_allclose(np.linalg.norm(got["normal"][hit].astype(np.float64), axis=1), 1.0, atol=1e-6)
     on_ray = rays[hit, 0:3].astype(np.float64) + rays[hit, 4:7].astype(np.float64) * got["t"][hit, None]
